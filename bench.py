@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            (N>1: launched by torch.distributed.run)
   python bench.py --impl reference --gpus N --steps K --warmup W
+  python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR   (+ the last timed step's outputs as DIR/*.npy)
 
 Workload (BASELINE.json configs[4], the largest single-GPU configuration): the synthetic sweep —
 10 000 videos x 2 000 steps of 1024-d bf16 features (30 000 frames at the dataset's 15x subsampling),
@@ -57,7 +58,15 @@ def parse_args():
                     help="videos per GPU (10000 = BASELINE config 5)")
     ap.add_argument("--e2e-videos", type=int, default=128)
     ap.add_argument("--cpu-seconds", type=float, default=15.0)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed (rank 0's videos) as DIR/<name>.npy: per-video and "
+                         "per-annotator F-scores of every video, frame scores and summaries of a fixed sample of videos")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs applies to --impl native")
+    return args
 
 
 def peaks():
@@ -348,6 +357,34 @@ def run_reference(args):
     except Exception as e:
         line["train"] = {"error": f"{type(e).__name__}: {e}"[:300]}
     print(json.dumps(line), flush=True)
+
+
+DUMP_VIDEOS = 256          # frame-level outputs of this many videos: 34 MB in all with the per-video arrays of 10 000 videos
+DUMP_LIMIT = 64 << 20
+
+
+def step_outputs(scores, batch, n_videos):
+    """Device copies of what a caller of the timed step receives: F-scores of every video (and of each of its
+    annotators), frame scores and frame-level summaries of a fixed, seeded sample of videos (indices in video_index)."""
+    import torch
+    idx = np.sort(np.random.default_rng(0).choice(n_videos, size=min(n_videos, DUMP_VIDEOS), replace=False))
+    d_idx = torch.from_numpy(idx).to(scores.device)
+    return {"video_index": torch.from_numpy(idx.astype(np.float64)),
+            "scores": scores.view(n_videos, N_STEPS).index_select(0, d_idx),
+            "summary": batch.summary[: n_videos * N_FRAMES].view(n_videos, N_FRAMES).index_select(0, d_idx),
+            "f_score_per_user": batch.f[: n_videos * N_USERS].view(n_videos, N_USERS).clone(),
+            "avg_f": batch.avg_f[:n_videos].clone(), "max_f": batch.max_f[:n_videos].clone()}
+
+
+def write_outputs(dirname, outputs):
+    arrays = {k: v.cpu().numpy() for k, v in outputs.items()}
+    assert all(a.dtype in (np.float32, np.float64) for a in arrays.values())
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT}-byte limit")
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(dirname, name + ".npy"), a)
 
 
 def make_features(n_videos, dev, seed):
@@ -824,9 +861,13 @@ def run_native(args):
     t_start.record(stream)
     for i in range(args.steps):
         evs[i][3].record(stream)
-        step(evs[i])
+        last = None                # each step's scores take the cached block the previous step's scores freed
+        last = step(evs[i])
     t_end.record(stream)
     barrier()
+    # the stages below reuse the batch's result buffers: the last timed step's results are copied first
+    outputs = step_outputs(last, batch, V) if args.dump_outputs and rank == 0 else None
+    del last
     clocks = sampler.stop() if rank == 0 else None
     if not model.check_status():
         raise RuntimeError("the fast scoring path left its checked value range inside the timed region")
@@ -1045,6 +1086,8 @@ def run_native(args):
             except Exception as e:
                 line["cpu_baseline"] = {"value": None, "unit": "videos/s", "cores": os.cpu_count(), "kind": "port",
                                         "sample": f"failed: {type(e).__name__}: {e}"[:300]}
+        if outputs is not None:
+            write_outputs(args.dump_outputs, outputs)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()

@@ -9,12 +9,12 @@ loudly when its CUDA library is missing.
 Parity status (see DESIGN.md "Oracle"):
   * eval path (upsample, segment pooling, summary vector, F-score): pinned
     against the reference's own Python, imported unmodified from
-    /root/reference in the build container (``oracle/ref_import.py``), with
+    a checkout named by $SMZ_REFERENCE_ROOT (``oracle/ref_import.py``), with
     golden vectors committed under ``tests/golden/``.
   * knapsack selection under ties: **parity unpinned** — the algorithm lives in
     the third-party dependency ``ortools==7.5.7466`` (summarizer/requirements.txt:11,
-    ``ortools/algorithms/knapsack_solver.cc``), which is neither vendored under
-    /root/reference nor installable here.  The restatement follows the published
+    ``ortools/algorithms/knapsack_solver.cc``), which the reference does not
+    vendor.  The restatement follows the published
     algorithm; optimal profit and feasibility are pinned against brute force.
   * VASNet / DSN scorers: pinned against the reference ``nn.Module``s imported
     unmodified (golden vectors under ``tests/golden/``).

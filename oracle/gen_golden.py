@@ -1,8 +1,8 @@
 """TEST INFRASTRUCTURE ONLY (see oracle/__init__.py).
 
 Generates the committed golden fixtures under tests/golden/ by running the UNMODIFIED reference
-(imported from /root/reference through oracle/ref_import.py) on seeded synthetic inputs.
-Run in the build container:   python -m oracle.gen_golden
+(imported from $SMZ_REFERENCE_ROOT through oracle/ref_import.py) on seeded synthetic inputs.
+With a reference checkout:   SMZ_REFERENCE_ROOT=<checkout> python -m oracle.gen_golden
 
   tests/golden/eval_golden.npz     inputs + reference outputs of generate_summary (knapsack via the
                                    restated OR-tools solver, and 'rank'), upsample, evaluate_summary

@@ -1,6 +1,6 @@
 """TEST INFRASTRUCTURE ONLY (see oracle/__init__.py).
 
-Golden vectors of the scorer models: the UNMODIFIED reference nn.Modules (imported from /root/reference
+Golden vectors of the scorer models: the UNMODIFIED reference nn.Modules (imported from $SMZ_REFERENCE_ROOT
 through oracle/ref_import.py) run on seeded weights and inputs on the CPU in float32.  The tests rebuild
 the same weights and inputs from the seeds, so only the outputs (and per-parameter checksums that prove
 the rebuilt weights are the reference's) are stored.   python -m oracle.gen_golden

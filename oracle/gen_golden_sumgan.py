@@ -1,5 +1,5 @@
 """TEST INFRASTRUCTURE — golden vectors for the SumGAN path, produced by the UNMODIFIED reference modules
-(summarizer/models/sumgan.py imported from /root/reference through oracle/ref_import.py), CPU float32.
+(summarizer/models/sumgan.py imported from $SMZ_REFERENCE_ROOT through oracle/ref_import.py), CPU float32.
 
     python oracle/gen_golden_sumgan.py        # writes tests/golden/sumgan_golden.npz
 

@@ -6,7 +6,7 @@ the CPU.  17 videos = 34 000 rows: more than one 32 768-row chunk of the packed 
 chunked, two-stream path with the fused exp / head epilogues on 8-video attention sub-chunks — exactly what bench.py
 times.  The features are regenerated from seeds by the tests; only the outputs are stored.
 
-    python -m oracle.gen_golden_sweep          (build container only: needs /root/reference)
+    python -m oracle.gen_golden_sweep          (needs SMZ_REFERENCE_ROOT, see oracle/ref_import.py)
 """
 import os
 

@@ -18,7 +18,7 @@ What is stored (tests/golden/train_golden.npz): per-epoch training losses (per o
 the six SumGAN log terms, the VAE pre-training loss, DSN rewards, the (corr, avg F, max F) Trainer.test returns after
 each epoch, train()'s return tuple, and initial / final values of sampled parameter entries (the Adam updates).
 
-    python -m oracle.gen_golden_train          (build container only: needs /root/reference)
+    python -m oracle.gen_golden_train          (needs SMZ_REFERENCE_ROOT, see oracle/ref_import.py)
 """
 import contextlib
 import logging

@@ -1,9 +1,10 @@
 """TEST INFRASTRUCTURE ONLY (see oracle/__init__.py).
 
-Imports the UNMODIFIED reference (sylvainma/Summarizer) from /root/reference in the
-build container so the oracle restatement can be validated against it and golden vectors
-can be generated (oracle/gen_golden.py).  /root/reference does not exist on the GPU box:
-nothing that runs there may call into this module (``available()`` is False there).
+Imports the UNMODIFIED reference (sylvainma/Summarizer) from a checkout of it, so the oracle
+restatement can be validated against it and golden vectors can be generated (oracle/gen_golden.py).
+The checkout is not part of this repository: $SMZ_REFERENCE_ROOT names its root directory (the one
+holding the reference's ``summarizer/`` package).  Without it ``available()`` is False and the tests
+marked ``reference`` skip.
 
 Two third-party modules the reference imports are absent from this image and are stubbed in
 ``sys.modules`` before import (SURVEY.md §8c):
@@ -21,11 +22,11 @@ import types
 
 import numpy as np
 
-REFERENCE_ROOT = "/root/reference"
+REFERENCE_ROOT = os.environ.get("SMZ_REFERENCE_ROOT", "")
 
 
 def available():
-    return os.path.isdir(os.path.join(REFERENCE_ROOT, "summarizer"))
+    return bool(REFERENCE_ROOT) and os.path.isdir(os.path.join(REFERENCE_ROOT, "summarizer"))
 
 
 class _DictDataset(dict):
@@ -84,8 +85,8 @@ def load():
     if _loaded:
         return _loaded["ns"]
     if not available():
-        raise RuntimeError("/root/reference is not present (GPU box?) — reference import is "
-                           "only possible in the build container")
+        raise RuntimeError("no reference checkout: set SMZ_REFERENCE_ROOT to the root of a sylvainma/Summarizer "
+                           "checkout")
     h5 = types.ModuleType("h5py")
     h5.File = DictFile
     sys.modules.setdefault("h5py", h5)

@@ -10,12 +10,13 @@ if ROOT not in sys.path:
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
-    config.addinivalue_line("markers", "reference: needs /root/reference (build container only)")
+    config.addinivalue_line("markers", "reference: needs a checkout of the reference project (SMZ_REFERENCE_ROOT)")
 
 
 def pytest_collection_modifyitems(config, items):
-    have_ref = os.path.isdir("/root/reference/summarizer")
-    skip_ref = pytest.mark.skip(reason="/root/reference not present")
+    from oracle import ref_import
+    have_ref = ref_import.available()
+    skip_ref = pytest.mark.skip(reason="SMZ_REFERENCE_ROOT does not name a checkout of the reference project")
     for item in items:
         if "reference" in item.keywords and not have_ref:
             item.add_marker(skip_ref)

@@ -91,10 +91,31 @@ def test_trainer_opens_synthetic_dataset_and_stages_keys(tmp_path):
     assert seq.shape == (300, 1, 1024) and float(target.min()) == 0.0 and float(target.max()) == 1.0
 
 
-@pytest.mark.reference
 def test_state_dict_matches_reference_modules():
+    """The drop-in VASNet keeps the reference module's state-dict layout, so a reference .pth loads unchanged.  Against
+    what the reference's own VASNet recorded: its key names and order and the initial values it drew at seeded entries
+    of each tensor (the entries depend on the tensor's size; tests/golden/train_golden.npz), and the per-parameter
+    checksums of the positional-embedding configurations (tests/golden/models_golden.npz).  With a reference checkout
+    (oracle/ref_import.py) also live: key lists, shapes and loading a reference state dict."""
+    from oracle import gen_golden_train as G
     from oracle import ref_import
+    from oracle.gen_golden_models import VASNET_CASES, build_vasnet, checksums
     from summarizer_b200.models.vasnet import VASNet
+    train = np.load(G.GOLDEN)
+    prefix = "vasnet/w0/"
+    names = [k[len(prefix):] for k in train.files if k.startswith(prefix)]      # stored in the reference's state_dict order
+    torch.manual_seed(G.RUNS["vasnet"]["seed"])
+    sampled = G.sampled_params(VASNet())
+    assert list(sampled) == names
+    for k in names:
+        np.testing.assert_array_equal(sampled[k], train[prefix + k], err_msg=k)
+    models = np.load(os.path.join(os.path.dirname(__file__), "golden", "models_golden.npz"))
+    pos_cases = [c for c in VASNET_CASES if "pos_embed" in c[4]]
+    assert pos_cases
+    for name, seed, _, _, kw, sharpen in pos_cases:
+        np.testing.assert_allclose(checksums(build_vasnet(VASNet, seed, kw, sharpen)), models[f"{name}/checksum"], rtol=1e-12)
+    if not ref_import.available():
+        return
     ref = ref_import.load()
     for kw in ({}, {"max_length": 32, "pos_embed": "simple"}):
         a, b = ref.vasnet.VASNet(**kw).state_dict(), VASNet(**kw).state_dict()

@@ -1,5 +1,5 @@
 """CPU tests of the oracle itself: it must agree with numpy, with the golden vectors generated
-from the unmodified reference, with the reference imported live (build container only) and, for
+from the unmodified reference, with the reference imported live (given a checkout, see oracle/ref_import.py) and, for
 the restated OR-tools solver, with brute force."""
 import itertools
 import os
