@@ -3,8 +3,8 @@
 Golden scores AT THE BENCHMARKED CONFIGURATION (BASELINE config 5 shapes): 17 videos x 2 000 steps x 1 024-d features that
 were rounded to bfloat16 (what the sweep stores), through the UNMODIFIED reference VASNet and DSN modules in float32 on
 the CPU.  17 videos = 34 000 rows: more than one 32 768-row chunk of the packed scorer, so the GPU test runs the
-chunked, two-stream path with the fused exp / head epilogues on 8-video attention sub-chunks — exactly what bench.py
-times.  The features are regenerated from seeds by the tests; only the outputs are stored.
+chunked, two-stream path with the fused exp / head epilogues — exactly what bench.py times.  The features are
+regenerated from seeds by the tests; only the outputs are stored.
 
     python -m oracle.gen_golden_sweep          (needs SMZ_REFERENCE_ROOT, see oracle/ref_import.py)
 """

@@ -4,6 +4,7 @@ Plain float32 PyTorch restatement of the reference scorers' forward passes, writ
 dict with the reference's key names so it can be fed with the product modules' parameters:
 
   vasnet_forward   models/vasnet.py:92-148 (eval mode, or training mode with explicit keep-masks)
+                   (vasnet_forward_packed: the same over a packed batch, video by video)
   dsn_forward      models/dsn.py:38-47     (nn.LSTM semantics restated step by step: gates i,f,g,o)
 
 Pinned by tests/test_oracle_models.py against tests/golden/models_golden.npz, i.e. against outputs of the
@@ -44,6 +45,13 @@ def vasnet_forward(sd, x, scale=None, eps=1e-6, aperture=None, ignore_self=False
         y = y * keep_h * 2.0                                     # :142
     y = F.layer_norm(y, (D,), sd["layer_norm.weight"], sd["layer_norm.bias"], eps)       # :143
     return torch.sigmoid(y @ sd["k2.weight"].t() + sd["k2.bias"]).reshape(T)             # :144-145
+
+
+def vasnet_forward_packed(sd, x, lengths, **kw):
+    """vasnet_forward over a packed batch x (sum T, 1024), one video at a time, in the dtype and on the device of x
+    (float64 on the GPU for the parity tests of the packed scorer) -> scores (sum T,)."""
+    sd = {k: v.to(x) for k, v in sd.items()}
+    return torch.cat([vasnet_forward(sd, xv, **kw) for xv in torch.split(x, list(lengths))])
 
 
 def lstm_direction(x, w_ih, w_hh, b_ih, b_hh, reverse=False):

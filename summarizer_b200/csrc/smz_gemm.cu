@@ -384,9 +384,9 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
                         for (int j = 0; j < 32; j++) if (n0 + j < g.N) x[j] += __bfloat162float(r[j]);
                     }
                 }
-                if (EPI != EPI_EXP && (flags & smz::GEMM_RELU)) {
+                if (EPI != EPI_EXP && (flags & smz::GEMM_RELU)) {    // NaN passes, as torch.relu (fmaxf would turn it into 0)
 #pragma unroll
-                    for (int j = 0; j < 32; j++) x[j] = fmaxf(x[j], 0.f);
+                    for (int j = 0; j < 32; j++) x[j] = x[j] < 0.f ? 0.f : x[j];
                 }
                 const bool f16 = EPI == EPI_PLAIN && (flags & smz::GEMM_OUT_F16) && n0 >= P.epi.f16_col0;     // warp-uniform
                 if (f16 && !(flags & smz::GEMM_LN_STATS)) {     // range check (with GEMM_LN_STATS the sum of squares does it)

@@ -21,7 +21,7 @@ static_assert(sizeof(GemmProblem) == 64, "GemmProblem layout");
 
 enum : int {
     GEMM_OUT_F32 = 1,    // C is float32 (default bf16)
-    GEMM_RELU = 2,       // max(x, 0) last
+    GEMM_RELU = 2,       // max(x, 0) last (NaN stays NaN)
     GEMM_RES_F32 = 4,    // residual is float32 (default bf16)
     GEMM_BIAS_M = 8,     // bias indexed by row m (default: by column n)
     GEMM_ROWSTATS = 16,  // per row and (n-tile, column half) slot: sum x, sum x^2, sum x * stat_w[n] of the epilogue

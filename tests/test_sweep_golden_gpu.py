@@ -1,8 +1,8 @@
 """GPU: the scorers AT THE BENCHMARKED CONFIGURATION against goldens of the unmodified reference modules
 (tests/golden/sweep_golden.npz, oracle/gen_golden_sweep.py): 17 videos x 2 000 steps, bfloat16 features, through
-``score_packed`` — for VASNet that is two 32 768-row chunks on the two internal streams, 8-video attention sub-chunks
-with the fused exp epilogue (no max subtraction), the fused head epilogue, i.e. the very path bench.py times, checked
-against the reference's float32 forward and not against itself."""
+``score_packed`` — for VASNet that is two row chunks (16 videos, then 1) on the two internal streams, one attention
+sub-chunk each (test_vasnet_plan_gpu.py asserts this plan) with the fused exp epilogue (no max subtraction), the fused
+head epilogue, i.e. the very path bench.py times, checked against the reference's float32 forward and not against itself."""
 import numpy as np
 import pytest
 import torch
