@@ -311,6 +311,51 @@ int smz_vasnet_backward(const void *x, int x_is_bf16, const int32_t *h_cu_seqlen
                         const uint8_t *drop_h, const float *scores, const float *dscores,
                         const smz_vasnet_grads *grads, void *ws, int64_t ws_bytes, void *stream);
 
+/* ---- Transformer scorer: replaces models/transformer.py Transformer.forward in eval mode (no autograd graph) ----------
+ * Fused variable-length multi-head attention, the encoder's hot path on its own:  out[:, h*128 : (h+1)*128] =
+ * softmax(Q_h K_h^T / sqrt(128)) V_h for every video and head, each video attending to all of its own frames and to no
+ * other video's.  qkv: bfloat16 [sum T, ld] device rows packed as nn.MultiheadAttention's in_proj output (Q columns
+ * [0, n_heads*128), K [n_heads*128, 2*n_heads*128), V after them; ld >= 3*n_heads*128, multiple of 8); out: bfloat16
+ * [sum T, ldo] (ldo >= n_heads*128, multiple of 8).  h_cu_seqlens as for smz_vasnet_forward.  head_dim must be 128
+ * (SMZ_ERR_UNSUPPORTED otherwise).  ws: smz_mha_workspace_bytes(n_videos) bytes of device memory (the work-unit table). */
+int smz_mha_workspace_bytes(int n_videos, int64_t *bytes);
+int smz_mha_forward(const void *qkv, int64_t ld, const int32_t *h_cu_seqlens, int n_videos, int n_heads, int head_dim,
+                    void *out, int64_t ldo, void *ws, int64_t ws_bytes, void *stream);
+
+/* One post-norm nn.TransformerEncoderLayer(d_model=1024, nhead=8, dim_feedforward=1024, relu): the parameters of
+ * transformer_encoder.layers.{i}.  Matrices are bfloat16 copies of the float32 weights ([out, in] row-major as torch
+ * stores them); vectors float32.  w_qkv [3072,1024] / b_qkv [3072] = self_attn.in_proj_weight / in_proj_bias (rows q, k,
+ * v); w_out = self_attn.out_proj; w1 / w2 = linear1 / linear2 [1024,1024]; norm1 / norm2 weights and biases (eps 1e-5). */
+typedef struct smz_transformer_layer {
+    const void *w_qkv;
+    const float *b_qkv;
+    const void *w_out;
+    const float *b_out;
+    const void *w1;
+    const float *b1;
+    const void *w2;
+    const float *b2;
+    const float *norm1_g, *norm1_b, *norm2_g, *norm2_b;
+} smz_transformer_layer;
+/* layers: HOST array of n_layers entries (read during the call only).  ln_g / ln_b / eps: the model's ONE layer_norm,
+ * applied as the encoder's final norm and again after relu(k1(.)).  k1_w bfloat16 [1024,1024], k1_b [1024];
+ * head_gw [1024] = ln_g * k2.weight, head_c [2] = {sum(ln_g * k2.weight), sum(ln_b * k2.weight) + k2.bias} (float32).
+ * more_residuals != 0: the head reads encoder_out + x. */
+typedef struct smz_transformer_params {
+    const smz_transformer_layer *layers;
+    const float *ln_g, *ln_b;
+    float eps;
+    int32_t more_residuals;
+    const void *k1_w;
+    const float *k1_b, *head_gw, *head_c;
+} smz_transformer_params;
+/* x: packed features [sum T, 1024] float32 (or bfloat16 when x_is_bf16), positional embeddings already added;
+ * scores: float32 [sum T].  ws: smz_transformer_workspace_bytes bytes. */
+int smz_transformer_workspace_bytes(const int32_t *h_cu_seqlens, int n_videos, int x_is_bf16, int64_t *bytes);
+int smz_transformer_forward(const void *x, int x_is_bf16, const int32_t *h_cu_seqlens, int n_videos,
+                            const smz_transformer_params *p, int n_layers, float *scores, void *ws, int64_t ws_bytes,
+                            void *stream);
+
 /* ---- DSN scorer: replaces models/dsn.py:38-47 DSN.forward (nn.LSTM(1024, 256, bidirectional) through
  *      cuDNN + Linear(512,1) + sigmoid) and, with smz_dsn_backward, its autograd graph ---------------------
  * Device pointers:

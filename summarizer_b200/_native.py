@@ -58,6 +58,10 @@ SIGNATURES = {
     "smz_vasnet_launch_count": (_I, [_P, _I, _I, _I, C.POINTER(C.c_int64)]),
     "smz_vasnet_forward": (_I, [_P, _I, _P, _I, _P, _I, _P, _P, _P, _P, _P, _L, _P]),
     "smz_vasnet_backward": (_I, [_P, _I, _P, _I, _P, _P, _P, _P, _P, _P, _P, _P, _L, _P]),
+    "smz_mha_workspace_bytes": (_I, [_I, C.POINTER(C.c_int64)]),
+    "smz_mha_forward": (_I, [_P, _L, _P, _I, _I, _I, _P, _L, _P, _L, _P]),
+    "smz_transformer_workspace_bytes": (_I, [_P, _I, _I, C.POINTER(C.c_int64)]),
+    "smz_transformer_forward": (_I, [_P, _I, _P, _I, _P, _I, _P, _P, _L, _P]),
     "smz_dsn_pack_whh": (_I, [_P, _P, _P, _P, _P]),
     "smz_dsn_workspace_bytes": (_I, [_I, _I, _I, _I, C.POINTER(C.c_int64)]),
     "smz_dsn_forward": (_I, [_P, _I, _P, _I, _P, _I, _P, _P, _L, _P]),

@@ -563,6 +563,10 @@ int make_map(CUtensorMap *m, const void *base, int64_t rows, int64_t cols, int64
 
 namespace smz {
 
+int make_bf16_map(CUtensorMap *m, const void *base, int64_t rows, int64_t cols, int64_t ld, int box_rows) {
+    return make_map(m, base, rows, cols, ld, box_rows);
+}
+
 int gemm_bf16_tn(const void *A, int64_t a_rows, int64_t a_cols, int64_t lda, const void *B, int64_t b_rows,
                  int64_t b_cols, int64_t ldb, const GemmProblem *d_probs, int n_probs, int total_tiles,
                  const GemmProblem &single, const GemmEpilogue &epi, cudaStream_t st) {

@@ -1,5 +1,7 @@
 // Host-side interface of the tcgen05 GEMM building block (smz_gemm.cu), shared by the scorer kernels.
 #pragma once
+#include <cuda.h>
+
 #include "smz_common.cuh"
 
 namespace smz {
@@ -94,5 +96,9 @@ int gemm_bf16_tn(const void *A, int64_t a_rows, int64_t a_cols, int64_t lda, con
 int gemm_bf16(bool a_mn, bool b_mn, const void *A, int64_t a_rows, int64_t a_cols, int64_t lda, const void *B,
               int64_t b_rows, int64_t b_cols, int64_t ldb, const GemmProblem *d_probs, int n_probs, int total_tiles,
               const GemmProblem &single, const GemmEpilogue &epi, cudaStream_t st);
+
+// TMA map of a bf16 [rows, cols] array (leading dimension ld elements): boxes of 64 columns x box_rows rows with the
+// 128-byte swizzle, the K-major operand layout the GEMM loads (smz_attn.cu loads its Q / K / V tiles with it too).
+int make_bf16_map(CUtensorMap *m, const void *base, int64_t rows, int64_t cols, int64_t ld, int box_rows);
 
 }  // namespace smz

@@ -240,7 +240,8 @@ softmax_kernel(const GemmProblem *__restrict__ probs, int n_probs, int total_row
 __global__ void __launch_bounds__(ROW_WARPS * 32)
 layernorm_kernel(const float *__restrict__ y, const uint8_t *__restrict__ keep, const float *__restrict__ g,
                  const float *__restrict__ b, float eps, int rows, __nv_bfloat16 *__restrict__ yn,
-                 float *__restrict__ mean, float *__restrict__ rstd, int64_t lo) {
+                 float *__restrict__ mean, float *__restrict__ rstd, int64_t lo, float *__restrict__ y32,
+                 const void *__restrict__ res, int res_bf16) {
     smz::pdl_trigger();
     smz::pdl_wait();
     const int lane = threadIdx.x & 31;
@@ -275,9 +276,20 @@ layernorm_kernel(const float *__restrict__ y, const uint8_t *__restrict__ keep, 
         const int c = lane * 4 + 128 * k;
         const float4 gg = *reinterpret_cast<const float4 *>(g + c);
         const float4 bb = *reinterpret_cast<const float4 *>(b + c);
-        const float o0 = (x[4 * k] - mu) * rs * gg.x + bb.x, o1 = (x[4 * k + 1] - mu) * rs * gg.y + bb.y;
-        const float o2 = (x[4 * k + 2] - mu) * rs * gg.z + bb.z, o3 = (x[4 * k + 3] - mu) * rs * gg.w + bb.w;
-        st_bf16x4(yn + (int64_t)r * kFeat + c, lo, o0, o1, o2, o3);
+        float o0 = (x[4 * k] - mu) * rs * gg.x + bb.x, o1 = (x[4 * k + 1] - mu) * rs * gg.y + bb.y;
+        float o2 = (x[4 * k + 2] - mu) * rs * gg.z + bb.z, o3 = (x[4 * k + 3] - mu) * rs * gg.w + bb.w;
+        if (res != nullptr) {
+            const int64_t ro = (int64_t)r * kFeat + c;
+            if (res_bf16) {
+                const __nv_bfloat16 *rb = reinterpret_cast<const __nv_bfloat16 *>(res) + ro;
+                o0 += __bfloat162float(rb[0]); o1 += __bfloat162float(rb[1]); o2 += __bfloat162float(rb[2]); o3 += __bfloat162float(rb[3]);
+            } else {
+                const float4 rr = *reinterpret_cast<const float4 *>(reinterpret_cast<const float *>(res) + ro);
+                o0 += rr.x; o1 += rr.y; o2 += rr.z; o3 += rr.w;
+            }
+        }
+        if (yn != nullptr) st_bf16x4(yn + (int64_t)r * kFeat + c, lo, o0, o1, o2, o3);
+        if (y32 != nullptr) *reinterpret_cast<float4 *>(y32 + (int64_t)r * kFeat + c) = make_float4(o0, o1, o2, o3);
     }
 }
 
@@ -633,10 +645,11 @@ int launch_softmax(const GemmProblem *d_probs, int n_probs, int total_rows, cons
 }
 
 int launch_layernorm(const float *y, const uint8_t *keep, const float *g, const float *b, float eps, int rows,
-                     __nv_bfloat16 *yn, float *mean, float *rstd, cudaStream_t st, int64_t lo) {
+                     __nv_bfloat16 *yn, float *mean, float *rstd, cudaStream_t st, int64_t lo, float *y32, const void *res,
+                     bool res_bf16) {
     if (rows <= 0) return SMZ_OK;
     SMZ_CUDA_CHECK(launch_pdl(layernorm_kernel, dim3((rows + ROW_WARPS - 1) / ROW_WARPS), dim3(ROW_WARPS * 32), 0, st, y, keep, g, b, eps, rows,
-                             yn, mean, rstd, lo));
+                             yn, mean, rstd, lo, y32, res, (int)res_bf16));
     return SMZ_OK;
 }
 

@@ -28,8 +28,11 @@ int launch_softmax(const GemmProblem *d_probs, int n_probs, int total_rows, cons
                    cudaStream_t st, const int *gate = nullptr, float *sum_slots = nullptr, int n_slots = 0, int64_t lo = 0);
 
 // yn = LayerNorm(2*keep*y or y) * g + b  (vasnet.py:136-137), rows of 1024; optional mean / rstd.
+// Optional: res (float32, or bf16 with res_bf16; rows of 1024) is added to the normalised row; y32 receives the result
+// in float32 as well (the transformer's residual stream); yn may then be NULL.
 int launch_layernorm(const float *y, const uint8_t *keep, const float *g, const float *b, float eps, int rows,
-                     __nv_bfloat16 *yn, float *mean, float *rstd, cudaStream_t st, int64_t lo = 0);
+                     __nv_bfloat16 *yn, float *mean, float *rstd, cudaStream_t st, int64_t lo = 0, float *y32 = nullptr,
+                     const void *res = nullptr, bool res_bf16 = false);
 
 // score = sigmoid(LayerNorm(2*keep*h or h) . w2 + b2)  (vasnet.py:142-145); h is post-ReLU float32.
 int launch_head(const float *h, const uint8_t *keep, const float *g, const float *b, float eps,
