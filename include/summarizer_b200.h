@@ -312,18 +312,19 @@ int smz_vasnet_backward(const void *x, int x_is_bf16, const int32_t *h_cu_seqlen
                         const smz_vasnet_grads *grads, void *ws, int64_t ws_bytes, void *stream);
 
 /* ---- Transformer scorer: replaces models/transformer.py Transformer.forward in eval mode (no autograd graph) ----------
- * Fused variable-length multi-head attention, the encoder's hot path on its own:  out[:, h*128 : (h+1)*128] =
- * softmax(Q_h K_h^T / sqrt(128)) V_h for every video and head, each video attending to all of its own frames and to no
- * other video's.  qkv: bfloat16 [sum T, ld] device rows packed as nn.MultiheadAttention's in_proj output (Q columns
- * [0, n_heads*128), K [n_heads*128, 2*n_heads*128), V after them; ld >= 3*n_heads*128, multiple of 8); out: bfloat16
- * [sum T, ldo] (ldo >= n_heads*128, multiple of 8).  h_cu_seqlens as for smz_vasnet_forward.  head_dim must be 128
+ * Fused variable-length multi-head attention, the encoder's hot path on its own:  out[:, h*D : (h+1)*D] =
+ * softmax(Q_h K_h^T / sqrt(D)) V_h for every video and head (D = head_dim), each video attending to all of its own frames
+ * and to no other video's.  qkv: bfloat16 [sum T, ld] device rows packed as nn.MultiheadAttention's in_proj output (Q
+ * columns [0, n_heads*D), K [n_heads*D, 2*n_heads*D), V after them; ld >= 3*n_heads*D, multiple of 8); out: bfloat16
+ * [sum T, ldo] (ldo >= n_heads*D, multiple of 8).  h_cu_seqlens as for smz_vasnet_forward.  head_dim must be 128 or 256
  * (SMZ_ERR_UNSUPPORTED otherwise).  ws: smz_mha_workspace_bytes(n_videos) bytes of device memory (the work-unit table). */
 int smz_mha_workspace_bytes(int n_videos, int64_t *bytes);
 int smz_mha_forward(const void *qkv, int64_t ld, const int32_t *h_cu_seqlens, int n_videos, int n_heads, int head_dim,
                     void *out, int64_t ldo, void *ws, int64_t ws_bytes, void *stream);
 
-/* One post-norm nn.TransformerEncoderLayer(d_model=1024, nhead=8, dim_feedforward=1024, relu): the parameters of
- * transformer_encoder.layers.{i}.  Matrices are bfloat16 copies of the float32 weights ([out, in] row-major as torch
+/* One post-norm nn.TransformerEncoderLayer(d_model=1024, nhead, dim_feedforward=1024, relu): the parameters of
+ * transformer_encoder.layers.{i}.  nhead is 8 for smz_transformer_forward and smz_sumgan_att_selector_params.n_heads for
+ * smz_sumgan_att_selector_forward.  Matrices are bfloat16 copies of the float32 weights ([out, in] row-major as torch
  * stores them); vectors float32.  w_qkv [3072,1024] / b_qkv [3072] = self_attn.in_proj_weight / in_proj_bias (rows q, k,
  * v); w_out = self_attn.out_proj; w1 / w2 = linear1 / linear2 [1024,1024]; norm1 / norm2 weights and biases (eps 1e-5). */
 typedef struct smz_transformer_layer {
@@ -355,6 +356,23 @@ int smz_transformer_workspace_bytes(const int32_t *h_cu_seqlens, int n_videos, i
 int smz_transformer_forward(const void *x, int x_is_bf16, const int32_t *h_cu_seqlens, int n_videos,
                             const smz_transformer_params *p, int n_layers, float *scores, void *ws, int64_t ws_bytes,
                             void *stream);
+
+/* ---- SumGAN-att selector: replaces models/sumgan_att.py Transformer.forward in eval mode (no autograd graph) ----------
+ * scores = sigmoid(out(layer_norm(TransformerEncoder(x)))).  layers: HOST array of n_layers encoder layers with n_heads
+ * heads of 1024 / n_heads (n_heads 4 or 8; SMZ_ERR_UNSUPPORTED otherwise, before any device work).  ln_g / ln_b / eps:
+ * the selector's layer_norm (the encoder's final norm); out_w [1024] / out_b [1]: out[0] = nn.Linear(1024, 1) (float32).
+ * x, h_cu_seqlens and scores as for smz_transformer_forward.  The work buffer is the same plan as the Transformer
+ * scorer's: ws: smz_transformer_workspace_bytes bytes. */
+typedef struct smz_sumgan_att_selector_params {
+    const smz_transformer_layer *layers;
+    int32_t n_heads;
+    const float *ln_g, *ln_b;
+    float eps;
+    const float *out_w, *out_b;
+} smz_sumgan_att_selector_params;
+int smz_sumgan_att_selector_forward(const void *x, int x_is_bf16, const int32_t *h_cu_seqlens, int n_videos,
+                                    const smz_sumgan_att_selector_params *p, int n_layers, float *scores,
+                                    void *ws, int64_t ws_bytes, void *stream);
 
 /* ---- DSN scorer: replaces models/dsn.py:38-47 DSN.forward (nn.LSTM(1024, 256, bidirectional) through
  *      cuDNN + Linear(512,1) + sigmoid) and, with smz_dsn_backward, its autograd graph ---------------------

@@ -62,6 +62,7 @@ SIGNATURES = {
     "smz_mha_forward": (_I, [_P, _L, _P, _I, _I, _I, _P, _L, _P, _L, _P]),
     "smz_transformer_workspace_bytes": (_I, [_P, _I, _I, C.POINTER(C.c_int64)]),
     "smz_transformer_forward": (_I, [_P, _I, _P, _I, _P, _I, _P, _P, _L, _P]),
+    "smz_sumgan_att_selector_forward": (_I, [_P, _I, _P, _I, _P, _I, _P, _P, _L, _P]),
     "smz_dsn_pack_whh": (_I, [_P, _P, _P, _P, _P]),
     "smz_dsn_workspace_bytes": (_I, [_I, _I, _I, _I, C.POINTER(C.c_int64)]),
     "smz_dsn_forward": (_I, [_P, _I, _P, _I, _P, _I, _P, _P, _L, _P]),

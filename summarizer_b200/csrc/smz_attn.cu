@@ -1,9 +1,13 @@
 // Fused variable-length multi-head attention (sm_100a): softmax(scale * Q_h K_h^T) V_h for every (video, head) of a
 // packed batch, without an attention mask inside a video and with no frame ever attending to another video's frames.
-// This is the attention of nn.TransformerEncoderLayer(d_model=1024, nhead=8) in eval mode (models/transformer.py).
+// This is the attention of nn.TransformerEncoderLayer(d_model=1024, nhead=8) (models/transformer.py, heads 128 wide) and
+// of nhead=4 (the SumGAN-att selector, models/sumgan_att.py, heads 256 wide) in eval mode.
 //
-// Input: the packed Q|K|V projection rows, bf16 [R, ld] (head h: Q columns [h*128, h*128+128), K at 1024 + h*128, V at
-// 2048 + h*128 for 8 heads), video v owning rows cu[v] .. cu[v+1]-1.  Output: bf16 [R, ldo], head h at column h*128.
+// Input: the packed Q|K|V projection rows, bf16 [R, ld] (head h: Q columns [h*HD, h*HD+HD), K at n_heads*HD + h*HD, V
+// at 2*n_heads*HD + h*HD), video v owning rows cu[v] .. cu[v+1]-1.  Output: bf16 [R, ldo], head h at column h*HD.
+// The kernel is a template on the head width HD (128 or 256); the key tile BKV is 128 keys for HD = 128 and 64 keys for
+// HD = 256, so that Q, P and a 2-stage K/V ring fit in shared memory (208 KB at HD = 256: Q 64 KB, P 16 KB, K and V
+// 32 KB per stage) and the two S buffers plus O fit the 512 TMEM columns.
 //
 // One work unit = one 128-row query tile of one (video, head).  Persistent grid; units are numbered longest video first
 // (the host sorts the videos), a CTA takes units blockIdx.x, blockIdx.x + gridDim.x, ...
@@ -12,12 +16,12 @@
 //              end -> -inf, online row max / row sum in fp32, P = exp2(s - max) as bf16 into shared memory (the
 //              tensor core's K-major 128-byte-swizzled layout); when the row max grows, the O accumulator row is
 //              rescaled in TMEM (tcgen05.ld / st).  After the last tile: O / l through a shared-memory pad to global.
-//   warp 4     TMA producer: Q once per unit, then K and V tiles of 128 keys into a 2-stage ring.  Video starts are not
-//              128-aligned: TMA takes any start row; rows of the next video are masked by the softmax, rows past the
-//              end of the array arrive zero-filled.
+//   warp 4     TMA producer: Q once per unit, then K and V tiles of BKV keys into a 2-stage ring.  Video starts are not
+//              aligned: TMA takes any start row; rows of the next video are masked by the softmax, rows past the end of
+//              the array arrive zero-filled.
 //   warp 5     MMA issuer: S_j = Q K_j^T into one of two TMEM score buffers (the QK^T of tile j+1 is issued before the
 //              P.V of tile j, so it overlaps the softmax of tile j), O += P_j V_j into a third TMEM region.
-// TMEM: S0 = columns [0,128), S1 = [128,256), O = [256,384) of a 512-column allocation.
+// TMEM: S0 = columns [0,BKV), S1 = [BKV,2*BKV), O = [2*BKV, 2*BKV+HD) of a 512-column allocation.
 // This is a true online softmax (running max subtraction): no range assumption on the logits.
 #include "smz_gemm.cuh"
 #include "smz_tc.cuh"
@@ -30,13 +34,26 @@ namespace {
 using namespace smztc;
 typedef __nv_bfloat16 bf16;
 
-constexpr int HD = 128;                   // head width (the only one supported)
-constexpr int BQ = 128, BKV = 128;        // query rows per unit, keys per tile
-constexpr int TILE_BYTES = BQ * HD * 2;   // 32 KB: one 128 x 128 bf16 tile
+constexpr int BQ = 128;                   // query rows per unit
 constexpr int STAGES = 2;
 constexpr int NUM_THREADS = 192;
-constexpr int SMEM_BYTES = (2 + 2 * STAGES) * TILE_BYTES + 256 + 1024;   // Q, P, K/V ring, barriers, alignment slack
 constexpr int TMEM_COLS = 512;
+
+// Tile shapes per head width.  Operands are stored as 64-column (128-byte) swizzled blocks: a K-major block of r rows
+// is r * 128 bytes, an MN-major V box (64 keys x 64 d-columns) is 8 KB.
+template <int HD>
+struct MhaShape {
+    static_assert(HD == 128 || HD == 256, "head width");
+    static constexpr int BKV = HD == 128 ? 128 : 64;        // keys per tile
+    static constexpr int DB = HD / 64;                       // 64-column blocks of a head
+    static constexpr int KB = BKV / 64;                      // 64-key blocks of a tile
+    static constexpr int Q_BYTES = BQ * HD * 2;
+    static constexpr int P_BYTES = BQ * BKV * 2;
+    static constexpr int KV_BYTES = BKV * HD * 2;            // one K or one V tile
+    static constexpr int SMEM_BYTES = Q_BYTES + P_BYTES + 2 * STAGES * KV_BYTES + 256 + 1024;   // + barriers, alignment slack
+    static_assert(2 * BKV + HD <= TMEM_COLS, "S double buffer and O exceed TMEM");
+    static_assert(SMEM_BYTES <= 227 * 1024, "shared memory");
+};
 
 struct MhaVideo { int32_t row0, T, unit0, qtiles; };
 static_assert(sizeof(MhaVideo) == 16, "MhaVideo layout");
@@ -62,15 +79,19 @@ struct UnitCursor {
     }
 };
 
+// tmQK: boxes of BKV rows x 64 columns (Q tiles are loaded as BQ / BKV boxes per column block); tmV: 64 x 64 boxes
+template <int HD>
 __global__ void __launch_bounds__(NUM_THREADS, 1)
 mha_fwd_kernel(const __grid_constant__ CUtensorMap tmQK, const __grid_constant__ CUtensorMap tmV, const MhaParams P) {
+    typedef MhaShape<HD> S;
+    constexpr int BKV = S::BKV, DB = S::DB, KB = S::KB, KV_BYTES = S::KV_BYTES;
     extern __shared__ uint8_t smem_raw[];
     uint8_t *smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);   // SWIZZLE_128B atoms
-    uint8_t *sQ = smem;
-    uint8_t *sP = smem + TILE_BYTES;
-    uint8_t *sK = smem + 2 * TILE_BYTES;                  // STAGES tiles
-    uint8_t *sV = sK + STAGES * TILE_BYTES;               // STAGES tiles: [key block kb][64 d-columns j] boxes of 8 KB
-    uint64_t *bars = reinterpret_cast<uint64_t *>(sV + STAGES * TILE_BYTES);
+    uint8_t *sQ = smem;                                   // [64-column block d] of BQ rows
+    uint8_t *sP = smem + S::Q_BYTES;                      // [64-key block kb] of BQ rows
+    uint8_t *sK = sP + S::P_BYTES;                        // STAGES tiles: [64-column block d] of BKV rows
+    uint8_t *sV = sK + STAGES * KV_BYTES;                 // STAGES tiles: [key block kb][64 d-columns j] boxes of 8 KB
+    uint64_t *bars = reinterpret_cast<uint64_t *>(sV + STAGES * KV_BYTES);
     uint64_t *q_full = bars, *q_empty = bars + 1;
     uint64_t *kv_full = bars + 2, *kv_empty = bars + 2 + STAGES;
     uint64_t *s_full = bars + 2 + 2 * STAGES, *s_empty = s_full + 2;
@@ -104,24 +125,28 @@ mha_fwd_kernel(const __grid_constant__ CUtensorMap tmQK, const __grid_constant__
             const int qcol = c.h * HD, kcol = P.n_heads * HD + c.h * HD, vcol = 2 * P.n_heads * HD + c.h * HD;
             mbar_wait(q_empty, (qn & 1u) ^ 1u);          // every QK^T of the previous unit has completed
             if (elect_one()) {
-                mbar_arrive_expect_tx(q_full, TILE_BYTES);
-                tma_load_2d(sQ, &tmQK, q_full, qcol, c.cur.row0 + c.qt * BQ);
-                tma_load_2d(sQ + TILE_BYTES / 2, &tmQK, q_full, qcol + 64, c.cur.row0 + c.qt * BQ);
+                mbar_arrive_expect_tx(q_full, S::Q_BYTES);
+#pragma unroll
+                for (int d = 0; d < DB; d++)
+#pragma unroll
+                    for (int rh = 0; rh < BQ / BKV; rh++)
+                        tma_load_2d(sQ + d * BQ * 128 + rh * BKV * 128, &tmQK, q_full, qcol + 64 * d,
+                                    c.cur.row0 + c.qt * BQ + rh * BKV);
             }
             __syncwarp();
             for (int j = 0; j < nk; j++) {
                 mbar_wait(&kv_empty[stage], phase ^ 1u);
                 if (elect_one()) {
                     const int r = c.cur.row0 + j * BKV;
-                    uint8_t *k = sK + stage * TILE_BYTES, *v = sV + stage * TILE_BYTES;
-                    mbar_arrive_expect_tx(&kv_full[stage], 2 * TILE_BYTES);
-                    tma_load_2d(k, &tmQK, &kv_full[stage], kcol, r);
-                    tma_load_2d(k + TILE_BYTES / 2, &tmQK, &kv_full[stage], kcol + 64, r);
+                    uint8_t *k = sK + stage * KV_BYTES, *v = sV + stage * KV_BYTES;
+                    mbar_arrive_expect_tx(&kv_full[stage], 2 * KV_BYTES);
 #pragma unroll
-                    for (int kb = 0; kb < 2; kb++)
+                    for (int d = 0; d < DB; d++) tma_load_2d(k + d * BKV * 128, &tmQK, &kv_full[stage], kcol + 64 * d, r);
 #pragma unroll
-                        for (int jn = 0; jn < 2; jn++)
-                            tma_load_2d(v + kb * 16384 + jn * 8192, &tmV, &kv_full[stage], vcol + 64 * jn, r + 64 * kb);
+                    for (int kb = 0; kb < KB; kb++)
+#pragma unroll
+                        for (int jn = 0; jn < DB; jn++)
+                            tma_load_2d(v + (kb * DB + jn) * 8192, &tmV, &kv_full[stage], vcol + 64 * jn, r + 64 * kb);
                 }
                 __syncwarp();
                 if (++stage == STAGES) { stage = 0; phase ^= 1u; }
@@ -140,13 +165,13 @@ mha_fwd_kernel(const __grid_constant__ CUtensorMap tmQK, const __grid_constant__
             mbar_wait(&s_empty[b], ((sn >> 1) & 1u) ^ 1u);
             mbar_wait(&kv_full[st], ph);
             tc_fence_after();
-            const uint32_t k_addr = smem_u32(sK + st * TILE_BYTES);
+            const uint32_t k_addr = smem_u32(sK + st * KV_BYTES);
             if (elect_one()) {
 #pragma unroll
-                for (int kb = 0; kb < 2; kb++) {
-                    const uint64_t qd = make_kmajor_sw128_desc(q_addr + kb * 16384), kd = make_kmajor_sw128_desc(k_addr + kb * 16384);
+                for (int d = 0; d < DB; d++) {
+                    const uint64_t qd = make_kmajor_sw128_desc(q_addr + d * BQ * 128), kd = make_kmajor_sw128_desc(k_addr + d * BKV * 128);
 #pragma unroll
-                    for (int k = 0; k < 4; k++) umma_bf16<false>(tS + b * BKV, qd + 2 * k, kd + 2 * k, idesc_s, (uint32_t)((kb | k) != 0));
+                    for (int k = 0; k < 4; k++) umma_bf16<false>(tS + b * BKV, qd + 2 * k, kd + 2 * k, idesc_s, (uint32_t)((d | k) != 0));
                 }
                 umma_commit<false>(&s_full[b]);
             }
@@ -168,11 +193,11 @@ mha_fwd_kernel(const __grid_constant__ CUtensorMap tmQK, const __grid_constant__
                 mbar_wait(p_full, pn & 1u);                           // P_j written, O rescaled
                 ++pn;
                 tc_fence_after();
-                const uint32_t v_addr = smem_u32(sV + stage * TILE_BYTES);
+                const uint32_t v_addr = smem_u32(sV + stage * KV_BYTES);
                 if (elect_one()) {
 #pragma unroll
-                    for (int kb = 0; kb < 2; kb++) {
-                        const uint64_t pd = make_kmajor_sw128_desc(p_addr + kb * 16384), vd = make_mnmajor_sw128_desc(v_addr + kb * 16384);
+                    for (int kb = 0; kb < KB; kb++) {
+                        const uint64_t pd = make_kmajor_sw128_desc(p_addr + kb * BQ * 128), vd = make_mnmajor_sw128_desc(v_addr + kb * DB * 8192);
 #pragma unroll
                         for (int k = 0; k < 4; k++) umma_bf16<false>(tO, pd + 2 * k, vd + 128 * k, idesc_o, (uint32_t)((j | kb | k) != 0));
                     }
@@ -200,16 +225,16 @@ mha_fwd_kernel(const __grid_constant__ CUtensorMap tmQK, const __grid_constant__
                 mbar_wait(&s_full[b], (sn >> 1) & 1u);
                 ++sn;
                 tc_fence_after();
-                uint32_t v[4][32];
+                uint32_t v[BKV / 32][32];
 #pragma unroll
-                for (int q = 0; q < 4; q++) tmem_ld32(tS + lane_off + b * BKV + 32 * q, v[q]);
+                for (int q = 0; q < BKV / 32; q++) tmem_ld32(tS + lane_off + b * BKV + 32 * q, v[q]);
                 tmem_ld_wait();
                 tc_fence_before();
                 mbar_arrive(&s_empty[b]);                  // the MMA warp may overwrite this S buffer
                 const int valid = T - j * BKV;             // keys of this tile inside the video (>= 1)
                 float mx = m_run;
 #pragma unroll
-                for (int q = 0; q < 4; q++)
+                for (int q = 0; q < BKV / 32; q++)
 #pragma unroll
                     for (int i = 0; i < 32; i++) {
                         const float s = (32 * q + i < valid) ? __uint_as_float(v[q][i]) * P.scale_log2 : -INFINITY;
@@ -225,7 +250,7 @@ mha_fwd_kernel(const __grid_constant__ CUtensorMap tmQK, const __grid_constant__
                     l_run *= alpha;
                     if (__any_sync(0xffffffffu, mx > m_run)) {      // warp-uniform: rescale the O rows of this warp
 #pragma unroll 1
-                        for (int q = 0; q < 4; q++) {
+                        for (int q = 0; q < HD / 32; q++) {
                             uint32_t o[32];
                             tmem_ld32(tO + lane_off + 32 * q, o);
                             tmem_ld_wait();
@@ -241,7 +266,7 @@ mha_fwd_kernel(const __grid_constant__ CUtensorMap tmQK, const __grid_constant__
                 // P row -> shared memory, K-major with the 128-byte swizzle: key block kb (64 keys) at kb * 16 KB, row r at
                 // r * 128 B, 16-byte chunk c (keys 8c..8c+7 of the block) at chunk position c ^ (r & 7)
 #pragma unroll
-                for (int q = 0; q < 4; q++) {
+                for (int q = 0; q < BKV / 32; q++) {
                     uint32_t pk[16];
 #pragma unroll
                     for (int i = 0; i < 32; i += 2) {
@@ -273,7 +298,7 @@ mha_fwd_kernel(const __grid_constant__ CUtensorMap tmQK, const __grid_constant__
             const int sub = lane >> 2, part = lane & 3;
             bf16 *obase = P.out + (int64_t)c.cur.row0 * P.ldo + c.h * HD + part * 8;
 #pragma unroll 1
-            for (int q = 0; q < 4; q++) {
+            for (int q = 0; q < HD / 32; q++) {
                 uint32_t o[32];
                 tmem_ld32(tO + lane_off + 32 * q, o);
                 tmem_ld_wait();
@@ -305,6 +330,31 @@ mha_fwd_kernel(const __grid_constant__ CUtensorMap tmQK, const __grid_constant__
     }
 }
 
+// Tensor maps, parameters and the launch of the HD-wide kernel (the table is already uploaded).
+template <int HD>
+int launch_mha(const void *qkv, int64_t rows, int64_t ld, int n_heads, MhaParams P, int64_t units, cudaStream_t st) {
+    typedef MhaShape<HD> S;
+    alignas(64) CUtensorMap mqk, mv;
+    const int64_t cols = 3LL * n_heads * HD;
+    int rc = smz::make_bf16_map(&mqk, qkv, rows, cols, ld, S::BKV);
+    if (rc != SMZ_OK) return rc;
+    rc = smz::make_bf16_map(&mv, qkv, rows, cols, ld, 64);
+    if (rc != SMZ_OK) return rc;
+    P.scale_log2 = 1.4426950408889634f / sqrtf((float)HD);
+    static bool attr_set[64] = {false};
+    int dev = 0;
+    SMZ_CUDA_CHECK(cudaGetDevice(&dev));
+    if (dev >= 0 && dev < 64 && !attr_set[dev]) {
+        SMZ_CUDA_CHECK(cudaFuncSetAttribute((const void *)mha_fwd_kernel<HD>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                            S::SMEM_BYTES));
+        attr_set[dev] = true;
+    }
+    const int grid = (int)std::min<int64_t>(units, (int64_t)smz::sm_count());
+    mha_fwd_kernel<HD><<<grid, NUM_THREADS, S::SMEM_BYTES, st>>>(mqk, mv, P);
+    SMZ_CUDA_CHECK(cudaGetLastError());
+    return SMZ_OK;
+}
+
 }  // namespace
 
 namespace smz {
@@ -313,14 +363,18 @@ int64_t mha_table_bytes(int n_videos) { return ((int64_t)n_videos * (int64_t)siz
 
 // Builds the unit table of videos [v0, v1) of h_cu (rows relative to h_cu[v0]), longest video first, uploads it to
 // d_table (mha_table_bytes(v1 - v0) bytes) and launches the kernel on qkv rows [0, rows).
-int mha_forward(const void *qkv, int64_t rows, int64_t ld, const int32_t *h_cu, int v0, int v1, int n_heads, void *out,
-                int64_t ldo, void *d_table, cudaStream_t st) {
+// head_dim: 128 or 256.
+int mha_forward(const void *qkv, int64_t rows, int64_t ld, const int32_t *h_cu, int v0, int v1, int n_heads, int head_dim,
+                void *out, int64_t ldo, void *d_table, cudaStream_t st) {
     const int n = v1 - v0;
     if (n <= 0) return SMZ_OK;
+    if (head_dim != 128 && head_dim != 256)
+        return fail(SMZ_ERR_UNSUPPORTED, "mha: head_dim %d is not supported (128 or 256)", head_dim);
     SMZ_REQUIRE(qkv && out && d_table && h_cu, "mha_forward: NULL pointer");
-    SMZ_REQUIRE(n_heads > 0 && ld >= 3LL * n_heads * HD && ldo >= (int64_t)n_heads * HD && (ldo & 7) == 0 &&
-                (reinterpret_cast<uintptr_t>(out) & 15) == 0,
-                "mha_forward: need ld >= 3 * n_heads * 128, ldo >= n_heads * 128, ldo % 8 == 0 and a 16-byte aligned output");
+    const int64_t w = (int64_t)n_heads * head_dim;
+    SMZ_REQUIRE(n_heads > 0 && ld >= 3 * w && ldo >= w && (ldo & 7) == 0 && (reinterpret_cast<uintptr_t>(out) & 15) == 0,
+                "mha_forward: need ld >= 3 * n_heads * head_dim, ldo >= n_heads * head_dim, ldo %% 8 == 0 and a 16-byte "
+                "aligned output");
     std::vector<int> order((size_t)n);
     for (int i = 0; i < n; i++) {
         order[i] = i;
@@ -344,12 +398,6 @@ int mha_forward(const void *qkv, int64_t rows, int64_t ld, const int32_t *h_cu, 
     SMZ_REQUIRE(rows >= h_cu[v1] - h_cu[v0], "mha_forward: fewer rows than the videos cover");
     int rc = upload_small(d_table, tab.data(), tab.size() * sizeof(MhaVideo), st);
     if (rc != SMZ_OK) return rc;
-    alignas(64) CUtensorMap mqk, mv;
-    const int64_t cols = 3LL * n_heads * HD;
-    rc = make_bf16_map(&mqk, qkv, rows, cols, ld, 128);
-    if (rc != SMZ_OK) return rc;
-    rc = make_bf16_map(&mv, qkv, rows, cols, ld, 64);
-    if (rc != SMZ_OK) return rc;
     MhaParams P;
     P.videos = reinterpret_cast<const MhaVideo *>(d_table);
     P.n_videos = n;
@@ -357,18 +405,8 @@ int mha_forward(const void *qkv, int64_t rows, int64_t ld, const int32_t *h_cu, 
     P.n_heads = n_heads;
     P.out = reinterpret_cast<bf16 *>(out);
     P.ldo = ldo;
-    P.scale_log2 = 1.4426950408889634f / sqrtf((float)HD);
-    static bool attr_set[64] = {false};
-    int dev = 0;
-    SMZ_CUDA_CHECK(cudaGetDevice(&dev));
-    if (dev >= 0 && dev < 64 && !attr_set[dev]) {
-        SMZ_CUDA_CHECK(cudaFuncSetAttribute((const void *)mha_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
-        attr_set[dev] = true;
-    }
-    const int grid = (int)std::min<int64_t>(units, (int64_t)sm_count());
-    mha_fwd_kernel<<<grid, NUM_THREADS, SMEM_BYTES, st>>>(mqk, mv, P);
-    SMZ_CUDA_CHECK(cudaGetLastError());
-    return SMZ_OK;
+    return head_dim == 128 ? launch_mha<128>(qkv, rows, ld, n_heads, P, units, st)
+                           : launch_mha<256>(qkv, rows, ld, n_heads, P, units, st);
 }
 
 }  // namespace smz
@@ -382,13 +420,14 @@ extern "C" int smz_mha_workspace_bytes(int n_videos, int64_t *bytes) {
 
 extern "C" int smz_mha_forward(const void *qkv, int64_t ld, const int32_t *h_cu_seqlens, int n_videos, int n_heads,
                                int head_dim, void *out, int64_t ldo, void *ws, int64_t ws_bytes, void *stream) {
-    if (head_dim != HD) return smz::fail(SMZ_ERR_UNSUPPORTED, "mha: head_dim %d is not supported (only 128)", head_dim);
+    if (head_dim != 128 && head_dim != 256)
+        return smz::fail(SMZ_ERR_UNSUPPORTED, "mha: head_dim %d is not supported (128 or 256)", head_dim);
     SMZ_REQUIRE(h_cu_seqlens != nullptr && n_videos > 0, "mha: empty batch");
     SMZ_REQUIRE(h_cu_seqlens[0] == 0, "mha: cu_seqlens[0] must be 0");
     SMZ_REQUIRE(ws != nullptr && ws_bytes >= smz::mha_table_bytes(n_videos), "mha: work buffer too small (%lld < %lld bytes)",
                 (long long)ws_bytes, (long long)smz::mha_table_bytes(n_videos));
     int rc = smz_device_check();
     if (rc != SMZ_OK) return rc;
-    return smz::mha_forward(qkv, h_cu_seqlens[n_videos], ld, h_cu_seqlens, 0, n_videos, n_heads, out, ldo, ws,
-                            (cudaStream_t)stream);
+    return smz::mha_forward(qkv, h_cu_seqlens[n_videos], ld, h_cu_seqlens, 0, n_videos, n_heads, head_dim, out, ldo,
+                            ws, (cudaStream_t)stream);
 }

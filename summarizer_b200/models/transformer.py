@@ -32,6 +32,36 @@ class TransformerParams(C.Structure):
                 ("head_c", C.c_void_p)]
 
 
+def encoder_params(layers):
+    """The parameters of nn.TransformerEncoderLayer modules in smz_transformer_layer order, flat (a weight cache's key)."""
+    return [t for L in layers for t in (L.self_attn.in_proj_weight, L.self_attn.in_proj_bias, L.self_attn.out_proj.weight,
+                                        L.self_attn.out_proj.bias, L.linear1.weight, L.linear1.bias, L.linear2.weight,
+                                        L.linear2.bias, L.norm1.weight, L.norm1.bias, L.norm2.weight, L.norm2.bias)]
+
+
+def f32(t):
+    return t.detach().float().contiguous()
+
+
+def b16(t):
+    return t.detach().to(torch.bfloat16).contiguous()
+
+
+def encoder_copies(layers):
+    """Per layer, the smz_transformer_layer tensors: bfloat16 copies of the matrices, float32 vectors."""
+    with torch.no_grad():
+        return [(b16(L.self_attn.in_proj_weight), f32(L.self_attn.in_proj_bias), b16(L.self_attn.out_proj.weight),
+                 f32(L.self_attn.out_proj.bias), b16(L.linear1.weight), f32(L.linear1.bias), b16(L.linear2.weight),
+                 f32(L.linear2.bias), f32(L.norm1.weight), f32(L.norm1.bias), f32(L.norm2.weight), f32(L.norm2.bias))
+                for L in layers]
+
+
+def layer_table(copies):
+    """The host array of smz_transformer_layer structs over encoder_copies(...); keep it alive for the call.  It is
+    rebuilt per call (plain tensors in the cache keep the module deep-copyable)."""
+    return (TransformerLayerParams * len(copies))(*(TransformerLayerParams(*(t.data_ptr() for t in ts)) for ts in copies))
+
+
 def sincos_table(max_length, width):
     """The fixed table of transformer.py:34-38: column i (even) sin(pos / 10000^(2i/width)), column i+1
     cos(pos / 10000^(2(i+1)/width)) — evaluated in float64 and rounded once, like the reference's numpy scalars."""
@@ -94,22 +124,12 @@ class Transformer(nn.Module):
         which reaches this module through ``_shadow_key``.  Only ``transformer_encoder.layers.*`` run: the top-level
         ``transformer_encoder_layer`` is a template the encoder deep-copied and is never read."""
         layers = list(self.transformer_encoder.layers)
-        ps = [t for L in layers for t in (L.self_attn.in_proj_weight, L.self_attn.in_proj_bias, L.self_attn.out_proj.weight,
-                                          L.self_attn.out_proj.bias, L.linear1.weight, L.linear1.bias, L.linear2.weight,
-                                          L.linear2.bias, L.norm1.weight, L.norm1.bias, L.norm2.weight, L.norm2.bias)]
+        ps = encoder_params(layers)
         ps += [self.layer_norm.weight, self.layer_norm.bias, self.k1.weight, self.k1.bias, self.k2.weight, self.k2.bias]
         key = tuple((p.data_ptr(), p._version) for p in ps) + (bool(self.more_residuals), float(self.epsilon))
         if self._shadow_key is None or key != self._shadow_key:
+            per_layer = encoder_copies(layers)
             with torch.no_grad():
-                def f32(t):
-                    return t.detach().float().contiguous()
-
-                def b16(t):
-                    return t.detach().to(torch.bfloat16).contiguous()
-                per_layer = [(b16(L.self_attn.in_proj_weight), f32(L.self_attn.in_proj_bias), b16(L.self_attn.out_proj.weight),
-                              f32(L.self_attn.out_proj.bias), b16(L.linear1.weight), f32(L.linear1.bias), b16(L.linear2.weight),
-                              f32(L.linear2.bias), f32(L.norm1.weight), f32(L.norm1.bias), f32(L.norm2.weight), f32(L.norm2.bias))
-                             for L in layers]
                 ln_g, ln_b = f32(self.layer_norm.weight), f32(self.layer_norm.bias)
                 w2, b2 = f32(self.k2.weight).reshape(-1), f32(self.k2.bias)
                 head_gw = (ln_g * w2).contiguous()
@@ -118,8 +138,7 @@ class Transformer(nn.Module):
                                     head_gw=head_gw, head_c=head_c)
             self._shadow_key = key
         sh = self._shadow
-        # the ctypes structs are rebuilt per call (plain tensors in the cache keep the module deep-copyable)
-        arr = (TransformerLayerParams * len(layers))(*(TransformerLayerParams(*(t.data_ptr() for t in ts)) for ts in sh["layers"]))
+        arr = layer_table(sh["layers"])
         st = TransformerParams(C.addressof(arr), sh["ln_g"].data_ptr(), sh["ln_b"].data_ptr(), float(self.epsilon),
                                int(bool(self.more_residuals)), sh["k1_w"].data_ptr(), sh["k1_b"].data_ptr(),
                                sh["head_gw"].data_ptr(), sh["head_c"].data_ptr())

@@ -29,8 +29,8 @@ class _NullWriter:
 
 
 def _model_registry():
-    """utils/config.py:68-77.  transformer scores on the library's kernels (its training stays on torch modules);
-    sumgan_att is a plain-torch passthrough module (outside the hot path, SURVEY.md §2.1; part of the drop-in surface, §8b)."""
+    """utils/config.py:68-77.  transformer and the sumgan_att selector score on the library's kernels (their training
+    stays on torch modules); sumgan_att's autoencoder is a plain-torch module (outside the hot path, SURVEY.md §2.1)."""
     from ..models.logistic import LogisticRegressionTrainer
     from ..models.rand import RandomTrainer
     from ..models.vasnet import VASNetTrainer
