@@ -1,10 +1,12 @@
 """TEST INFRASTRUCTURE ONLY (see oracle/__init__.py).
 
-Python restatement of the inference launch plan of ``smz_vasnet_forward`` (``make_plan`` in
-summarizer_b200/csrc/smz_vasnet.cu): how a packed batch is split into row chunks, attention sub-chunks and lanes,
-and the work-buffer size that follows.  tests/test_vasnet_plan_gpu.py pins it against the library's own
-``smz_vasnet_launch_count`` / ``smz_vasnet_workspace_bytes`` (host-only entry points, no device needed) and then uses
-it to assert that every batch a GPU test runs reaches the plan structure it is meant to cover.
+Python restatement of the launch plan of ``smz_vasnet_forward`` (``make_plan`` in summarizer_b200/csrc/smz_vasnet.cu):
+for inference, how a packed batch is split into row chunks, attention sub-chunks and lanes; for training
+(``smz_vasnet_forward(training=1)`` + ``smz_vasnet_backward``), the per-video regions of the work buffer; and the
+work-buffer size that follows.  tests/test_vasnet_plan_gpu.py (inference) and tests/test_vasnet_train_plan_gpu.py
+(training) pin it against the library's own ``smz_vasnet_launch_count`` / ``smz_vasnet_workspace_bytes`` (host-only
+entry points, no device needed) and then use it to assert that every batch a GPU test runs reaches the plan structure
+it is meant to cover.
 """
 from typing import List, NamedTuple
 
@@ -14,6 +16,7 @@ FEAT = 1024                 # kFeat
 GEMM_BN = 256               # smz::GEMM_BN: columns per GEMM tile, two row-sum slots per tile
 LN_SLOTS = 2 * FEAT // GEMM_BN
 PROBLEM_BYTES = 64          # sizeof(smz::GemmProblem)
+ROW_WARPS = 8               # warps (one row each per pass) of a CTA of the row kernels, smz_rows.cu
 
 
 def up(x, m):
@@ -90,3 +93,57 @@ def workspace_bytes(lengths, x_bf16, budget=LOGIT_BUDGET):
         R * LN_SLOTS * 3 * 4))              # LayerNorm sums
     lanes = 2 if len(chunks) > 1 else 1
     return lanes * lane + up(len(lengths) * 2 * PROBLEM_BYTES, 1024)
+
+
+# ---- training ------------------------------------------------------------------------------------------------------
+class TrainChunk(NamedTuple):
+    v: int          # the video (a training chunk holds exactly one, with one attention sub-chunk)
+    row0: int       # first row in the row-wise buffers (the packed row of the video)
+    rows: int
+    vt_off: int     # element offset of the video's V^T (and dV^T) region, [1024, up(T, 8)]
+    lg_off: int     # element offset of the video's logits (P, alpha, dP, dS) region, [T, ld]
+    ld: int         # row length of that logits region: up(T + 7, 64)
+
+
+def training_plan(lengths):
+    """Chunks of a training call: every video is a chunk of its own and owns a region of each buffer."""
+    assert len(lengths) > 0 and all(T > 0 for T in lengths)
+    out, row0, vt, lg = [], 0, 0, 0
+    for v, T in enumerate(lengths):
+        ld = up(T + 7, 64)
+        out.append(TrainChunk(v, row0, T, vt, lg, ld))
+        row0, vt, lg = row0 + T, vt + FEAT * up(T, 8), lg + T * ld
+    return out
+
+
+def training_launch_count(lengths, x_bf16):
+    """Kernel launches of smz_vasnet_forward(training=1): per video [cvt] QK Vt out layernorm k1 head + logits, softmax,
+    alpha.V (one sub-chunk)."""
+    return len(lengths) * ((0 if x_bf16 else 1) + 6 + 3)
+
+
+def training_workspace_bytes(lengths, x_bf16, split=False):
+    """Work-buffer bytes of a training call (forward and backward share it).  split: the float32-accurate mode
+    (SMZ_VASNET_SPLIT), whose second half holds the lo planes at the same offsets."""
+    plan = training_plan(lengths)
+    R = up(sum(lengths), 8)
+    VT = sum(FEAT * up(c.rows, 8) for c in plan)
+    LG = sum(c.rows * c.ld for c in plan)
+    total = sum(up(b, 1024) for b in (
+        0 if x_bf16 else R * FEAT * 2,      # bf16 copy of float32 features
+        R * 2 * FEAT * 2,                   # Q | K rows
+        VT * 2,                             # V^T of every video
+        R * FEAT * 2, R * FEAT * 4, R * FEAT * 2, R * FEAT * 4,     # o, y, yn, h
+        LG * 4, LG * 2, LG * 2,             # fp32 logits (dP in the backward), probabilities, dropped-out probabilities
+        len(lengths) * 2 * PROBLEM_BYTES,   # GEMM problem tables
+        len(lengths) * 8,                   # offsets of the attention keep-masks
+        R * 4 * 4,                          # mean / rstd of both LayerNorms
+        R * FEAT * 2, R * FEAT * 4, R * FEAT * 2, R * FEAT * 4, R * FEAT * 2,   # dh, dyn, dy, dy float32, dO
+        R * 2 * FEAT * 2, VT * 2, LG * 2))  # dQ | dK, dV^T, dS
+    return 2 * total if split else total
+
+
+def row_grid_rows(sm_count):
+    """Rows one pass of the capped backward row kernels covers (launch_head_bwd / launch_layernorm_bwd: at most
+    2 * sm_count CTAs of ROW_WARPS warps, one row per warp); longer videos make every warp loop over rows."""
+    return 2 * sm_count * ROW_WARPS
