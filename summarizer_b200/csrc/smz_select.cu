@@ -23,6 +23,8 @@
 #include <limits.h>
 #include <stdlib.h>
 
+#include <mutex>
+
 namespace {
 
 using namespace smzdev;
@@ -132,7 +134,7 @@ constexpr int POOL_REG_THREADS = 256;
 
 struct RegularFrames {   // upsample of a regular pick grid: scores staged in shared memory (zero-filled past n_scores)
     const float *sc;
-    uint32_t magic;      // floor(2^32 / stride) + 1: f / stride == umulhi(f, magic) for f, stride < 65536
+    uint32_t magic;      // floor(2^32 / stride) + 1: f / stride == umulhi(f, magic) for f < 65536, 2 <= stride < 65536
     int last;            // index of the last interval
     __device__ __forceinline__ float at(int f) const { return sc[min((int)__umulhi((uint32_t)f, magic), last)]; }
 };
@@ -153,14 +155,15 @@ __device__ void pool_regular_video(const smz_video_desc &d, int v, const float *
     const int n_int = n_bound - 1;                                   // intervals [bound(i), bound(i+1))
     if (tid == 0 && n_int > d.n_scores + 1) atomicOr(status + v, SMZ_STATUS_INTERVALS);
     const int stride = n_picks >= 2 ? __ldg(pk + 1) - __ldg(pk) : n_frames;
-    int ok = n_picks >= 1 && n_int >= 1 && n_int <= max_intervals && stride >= 1 && stride < 65536 && n_frames < 65536;
+    // stride 1 (a pick on every frame) takes the cursor walk: 2^32 / 1 does not fit the 32-bit multiplier
+    int ok = n_picks >= 1 && n_int >= 1 && n_int <= max_intervals && stride >= 2 && stride < 65536 && n_frames < 65536;
     for (int i = tid; i < n_picks && ok; i += NT) ok = __ldg(pk + i) == i * stride;
     for (int i = tid; i < n_int && i < max_intervals; i += NT) s_sc[i] = i < d.n_scores ? __ldg(sc + i) : 0.f;
     ok = __syncthreads_and(ok);
     const int lane = tid & 31, gl = lane & 7, lane0 = lane & ~7;
     const unsigned gmask = 0xffu << lane0;
     const int vlim = value_limit(n);
-    RegularFrames reg{s_sc, (uint32_t)(0x100000000ull / (uint32_t)max(stride, 1)) + 1u, n_int - 1};
+    RegularFrames reg{s_sc, (uint32_t)(0x100000000ull / (uint32_t)max(stride, 2)) + 1u, n_int - 1};
     FrameCursor cur;
     if (!ok) cur.init(sc, pk, d.n_scores, n_picks, n_frames);
     // Segments are handed to the 8-lane groups sorted by the SHAPE of their pairwise-summation tree (one block up to
@@ -1209,11 +1212,15 @@ constexpr int kQueueHead32 = 1 + 2 * ORDER_BUCKETS, kFallback = kQueueHead32 + 1
 static int64_t queue_bytes(int n_videos) { return (int64_t)(kQueueInts + 2 * (int64_t)n_videos) * 4 + 256; }
 
 // cudaFuncSetAttribute + occupancy query once per (device, kernel, dynamic shared memory): the plan is rebuilt on every
-// call and these two driver calls would otherwise dominate its host time
+// call and these two driver calls would otherwise dominate its host time.  Callers may plan from several host threads
+// at once (ctypes releases the GIL): the table and the attribute it tracks change under one lock, so one thread cannot
+// lower a kernel's shared-memory limit below what another has planned a launch with.
 static int cached_occupancy(const void *fn, int threads, int smem_bytes, int *per_sm) {
     struct Entry { int dev; const void *fn; int smem, per_sm; };
+    static std::mutex mu;
     static Entry table[96];
     static int used = 0;
+    std::lock_guard<std::mutex> lock(mu);
     int dev = 0;
     SMZ_CUDA_CHECK(cudaGetDevice(&dev));
     int attr = -1;                       // largest dynamic size this kernel's attribute was raised to on this device
@@ -1222,11 +1229,15 @@ static int cached_occupancy(const void *fn, int threads, int smem_bytes, int *pe
         if (table[i].smem == smem_bytes) { *per_sm = table[i].per_sm; return SMZ_OK; }
         if (table[i].smem > attr) attr = table[i].smem;
     }
-    if (smem_bytes > attr)               // only ever raised, so launches planned from older entries stay valid
+    if (used >= 96) {                    // a full table no longer knows every size the attribute was raised to: ask
+        cudaFuncAttributes fa;
+        SMZ_CUDA_CHECK(cudaFuncGetAttributes(&fa, fn));
+        attr = fa.maxDynamicSharedSizeBytes;
+    }
+    if (smem_bytes > attr)               // only ever raised, so launches planned earlier (on any thread) stay valid
         SMZ_CUDA_CHECK(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
     SMZ_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(per_sm, fn, threads, smem_bytes));
-    if (used < 96) table[used++] = Entry{dev, fn, smem_bytes, *per_sm};     // callers hold the GIL / own the stream
-    else SMZ_CUDA_CHECK(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes > attr ? smem_bytes : attr));
+    if (used < 96) table[used++] = Entry{dev, fn, smem_bytes, *per_sm};
     return SMZ_OK;
 }
 
