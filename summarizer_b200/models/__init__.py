@@ -18,6 +18,7 @@ from .. import synthetic
 from ..batch import VideoBatch
 from ..rankcorr import CorrBatch
 from ..utils.eval import evaluate_scores, evaluate_summary, generate_scores, generate_summary  # noqa: F401 (reference surface)
+from ._packed import NativeModule
 
 
 def h5_file(path, mode):
@@ -245,14 +246,20 @@ class Trainer:
         return self._fold_eval[tag]
 
     # ---- evaluation -------------------------------------------------------------------------------
+    def _packed_scorer(self):
+        """The module whose ``score_packed`` scores all test videos in ONE call (ragged batch), or None to run the
+        model's forward once per video."""
+        return None
+
     def _score_keys(self, keys):
         """Model scores of several videos -> list of (T,) float32 device tensors."""
-        out = []
+        scorer = self._packed_scorer()
         with torch.no_grad():
-            for key in keys:
-                seq, _ = self._video_tensors(key)
-                out.append(self.model(self._model_input(seq)).reshape(-1).float())
-        return out
+            if scorer is not None:
+                feats = [self._video_tensors(k)[0][:, 0] for k in keys]
+                lengths = [f.shape[0] for f in feats]
+                return list(torch.split(scorer.score_packed(torch.cat(feats), lengths), lengths))
+            return [self.model(self._model_input(self._video_tensors(k)[0])).reshape(-1).float() for k in keys]
 
     def test(self, fold):
         """Test model on test_keys -> (avg_corr, (avg_f_score, max_f_score))  (models/__init__.py:40-58)"""
@@ -355,10 +362,8 @@ class Trainer:
     def _invalidate_shadows(self):
         """Drop the modules' cached bf16 / packed weight copies (they are rebuilt on the next call)."""
         for m in self.model.modules():
-            if hasattr(m, "_shadow_key"):
-                m._shadow_key = None
-            if hasattr(m, "_cache") and hasattr(m._cache, "_store"):
-                m._cache._store.clear()
+            if isinstance(m, NativeModule):
+                m._cache.clear()
 
     # ---- supervised loop shared by the MSE-trained scorers (vasnet.py:171-238, logistic.py:42-112) ---
     def _train_supervised(self, fold, optimizer_params=None):

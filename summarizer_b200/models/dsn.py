@@ -9,13 +9,14 @@ Parameters live in an ``nn.LSTM`` / ``nn.Sequential`` pair exactly like the refe
 never executed.  Only the default configuration the reference trainer builds (LSTM cell, 1 layer, hidden 256,
 dsn.py:58) is implemented; there is no CPU fallback."""
 import ctypes as C
+import functools
 
 import numpy as np
 import torch
 import torch.nn as nn
 
 from .. import _native as N
-from .vasnet import _cu_seqlens, _Workspace
+from ._packed import NativeModule, Workspace, packed_input, score_sequences, workspace_bytes
 
 
 class DsnParams(C.Structure):
@@ -23,7 +24,7 @@ class DsnParams(C.Structure):
     _fields_ = [(k, C.c_void_p) for k in ("w_ih", "bias", "whh_packed", "whh_t_packed", "w_out", "b_out")]
 
 
-class DSN(nn.Module):
+class DSN(NativeModule):
     """Deep Summarization Network"""
 
     def __init__(self, input_size=1024, hidden_size=256, num_layers=1, cell="lstm"):
@@ -34,7 +35,7 @@ class DSN(nn.Module):
                                       "LSTM cell, 1024-d input, hidden size 256, one layer (dsn.py:58)")
         self.rnn = nn.LSTM(input_size, hidden_size, num_layers=num_layers, bidirectional=True)
         self.out = nn.Sequential(nn.Linear(hidden_size * 2, 1), nn.Sigmoid())
-        self._shadow, self._shadow_key, self._ws = None, None, _Workspace()
+        self._ws = Workspace()
 
     def _params(self):
         r, o = self.rnn, self.out[0]
@@ -42,39 +43,28 @@ class DSN(nn.Module):
                 r.bias_ih_l0_reverse, r.bias_hh_l0_reverse, o.weight, o.bias)
 
     def _weights(self, training=False):
-        """bf16 / packed shadow copies for the kernels.  A training forward always rebuilds them and leaves the cache
-        dirty (fused optimizers update parameters without bumping ``Tensor._version``); inference calls reuse them
-        until a parameter's version / storage changes or a training forward happened in between."""
-        ps = self._params()
-        key = tuple((p.data_ptr(), p._version) for p in ps)
-        if training or self._shadow_key is None or key != self._shadow_key:
-            wih_f, whh_f, bih_f, bhh_f, wih_b, whh_b, bih_b, bhh_b, w_out, b_out = ps
-            with torch.no_grad():
-                dev = wih_f.device
-                sh = dict(w_ih=torch.cat([wih_f, wih_b], 0).to(torch.bfloat16).contiguous(),
-                          bias=torch.cat([bih_f + bhh_f, bih_b + bhh_b]).float().contiguous(),
-                          whh=torch.empty(2 * 8 * 64 * 256, dtype=torch.int32, device=dev),
-                          whh_t=torch.empty(2 * 8 * 64 * 256, dtype=torch.int32, device=dev),
-                          w_out=w_out.float().reshape(-1).contiguous(), b_out=b_out.float().contiguous())
-                N.check(N.lib().smz_dsn_pack_whh(N.ptr(whh_f.float().contiguous()), N.ptr(whh_b.float().contiguous()),
-                                                 N.ptr(sh["whh"]), N.ptr(sh["whh_t"]), N.current_stream()))
-            self._shadow, self._shadow_key = sh, (None if training else key)
-        sh = self._shadow
-        st = DsnParams(*(sh[k].data_ptr() for k in ("w_ih", "bias", "whh", "whh_t", "w_out", "b_out")))
-        return sh, st
+        """The kernels' weight copies (cached in ``self._cache``; a training forward rebuilds them) and the parameter
+        struct over them."""
+        sh = self._cache.get(self._params(), self._build_weights, fresh=training)
+        return sh, DsnParams(*(sh[k].data_ptr() for k in ("w_ih", "bias", "whh", "whh_t", "w_out", "b_out")))
+
+    def _build_weights(self):
+        wih_f, whh_f, bih_f, bhh_f, wih_b, whh_b, bih_b, bhh_b, w_out, b_out = self._params()
+        dev = wih_f.device
+        sh = dict(w_ih=torch.cat([wih_f, wih_b], 0).to(torch.bfloat16).contiguous(),
+                  bias=torch.cat([bih_f + bhh_f, bih_b + bhh_b]).float().contiguous(),
+                  whh=torch.empty(2 * 8 * 64 * 256, dtype=torch.int32, device=dev),
+                  whh_t=torch.empty(2 * 8 * 64 * 256, dtype=torch.int32, device=dev),
+                  w_out=w_out.float().reshape(-1).contiguous(), b_out=b_out.float().contiguous())
+        N.check(N.lib().smz_dsn_pack_whh(N.ptr(whh_f.float().contiguous()), N.ptr(whh_b.float().contiguous()),
+                                         N.ptr(sh["whh"]), N.ptr(sh["whh_t"]), N.current_stream()))
+        return sh
 
     def score_packed(self, x, lengths):
         """Inference over a ragged batch: x packed [sum T, 1024] (float32 / bfloat16) -> probs [sum T]."""
-        N.require_device()
-        if x.dtype not in (torch.float32, torch.bfloat16):
-            x = x.float()
-        x = x.contiguous()
-        cu = _cu_seqlens(lengths)
+        x, cu, is_bf16 = packed_input(x, lengths, 1024)
         _, st = self._weights()
-        is_bf16 = int(x.dtype == torch.bfloat16)
-        nbytes = C.c_int64(0)
-        N.check(N.lib().smz_dsn_workspace_bytes(int(cu[-1]), len(lengths), 0, is_bf16, C.byref(nbytes)))
-        ws = self._ws.get(nbytes.value, x.device)
+        ws = self._ws.get(workspace_bytes(N.lib().smz_dsn_workspace_bytes, int(cu[-1]), len(lengths), 0, is_bf16), x.device)
         probs = torch.empty(x.shape[0], dtype=torch.float32, device=x.device)
         N.check(N.lib().smz_dsn_forward(N.ptr(x), is_bf16, cu.ctypes.data_as(C.c_void_p), len(lengths), C.byref(st), 0,
                                         N.ptr(probs), N.ptr(ws), ws.numel(), N.current_stream()))
@@ -87,16 +77,12 @@ class DSN(nn.Module):
         Output
           probs: (seq_len, batch_size, 1)
         """
-        seq_len, batch_size, _ = x.shape
         if not x.is_cuda:
             raise N.NativeError("summarizer_b200.DSN runs on a CUDA (sm_100a) device only; move the input with .cuda()")
-        packed = x.permute(1, 0, 2).reshape(batch_size * seq_len, -1)
         if torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters()):
             from .dsn_autograd import dsn_apply
-            p = dsn_apply(self, packed, [seq_len] * batch_size)
-        else:
-            p = self.score_packed(packed, [seq_len] * batch_size)
-        return p.view(batch_size, seq_len, 1).permute(1, 0, 2)
+            return score_sequences(functools.partial(dsn_apply, self), x)
+        return score_sequences(self.score_packed, x)
 
 
 
@@ -110,9 +96,7 @@ def compute_rewards(seq, actions, far_sim=False, temp_dist_thre=20, workspace=No
     seq = seq.detach().reshape(-1, 1024).float().contiguous()
     act = actions.detach().reshape(actions.shape[0], -1).to(torch.uint8).contiguous()
     E, T = act.shape
-    nbytes = C.c_int64(0)
-    N.check(N.lib().smz_dsn_reward_workspace_bytes(T, E, C.byref(nbytes)))
-    ws = (workspace or _Workspace()).get(nbytes.value, seq.device)
+    ws = (workspace or Workspace()).get(workspace_bytes(N.lib().smz_dsn_reward_workspace_bytes, T, E), seq.device)
     rewards = torch.empty(E, dtype=torch.float32, device=seq.device)
     N.check(N.lib().smz_dsn_reward(N.ptr(seq), T, N.ptr(act), E, int(temp_dist_thre), int(bool(far_sim)), N.ptr(rewards),
                                    N.ptr(ws), ws.numel(), N.current_stream()))
@@ -177,7 +161,7 @@ class DSNTrainer(Trainer):
         self.far_sim = bool(ep.get("far_sim", False))
         self.temp_dist_thre = int(ep.get("temp_dist_thre", 20))
         self.sup = bool(ep.get("sup", False))
-        self._reward_ws = _Workspace()
+        self._reward_ws = Workspace()
         return DSN()
 
     def _draw_actions(self, probs):
@@ -189,12 +173,8 @@ class DSNTrainer(Trainer):
         """One episode (reference signature, dsn.py:185): seq (T,1,1024), actions (T,1,1) -> scalar tensor."""
         return compute_rewards(seq.reshape(-1, 1024), actions.reshape(1, -1), far_sim, temp_dist_thre, self._reward_ws)[0]
 
-    def _score_keys(self, keys):
-        feats = [self._video_tensors(k)[0][:, 0] for k in keys]
-        lengths = [f.shape[0] for f in feats]
-        with torch.no_grad():
-            packed = self.model.score_packed(torch.cat(feats), lengths)
-        return list(torch.split(packed, lengths))
+    def _packed_scorer(self):
+        return self.model
 
     def train(self, fold):
         import random

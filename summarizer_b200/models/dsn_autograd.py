@@ -4,8 +4,8 @@ import ctypes as C
 import torch
 
 from .. import _native as N
+from ._packed import packed_input, workspace_bytes
 from .dsn import DsnParams
-from .vasnet import _cu_seqlens
 
 
 class DsnGrads(C.Structure):
@@ -16,16 +16,10 @@ class DsnGrads(C.Structure):
 class _DsnFunction(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, module, lengths, *params):
-        N.require_device()
-        x = x.contiguous()
-        if x.dtype not in (torch.float32, torch.bfloat16):
-            x = x.float()
-        cu = _cu_seqlens(lengths)
-        is_bf16 = int(x.dtype == torch.bfloat16)
+        x, cu, is_bf16 = packed_input(x, lengths, 1024)
         sh, st = module._weights(training=True)
-        nbytes = C.c_int64(0)
-        N.check(N.lib().smz_dsn_workspace_bytes(int(cu[-1]), len(lengths), 1, is_bf16, C.byref(nbytes)))
-        ws = torch.empty(max(nbytes.value, 1024), dtype=torch.uint8, device=x.device)
+        nbytes = workspace_bytes(N.lib().smz_dsn_workspace_bytes, int(cu[-1]), len(lengths), 1, is_bf16)
+        ws = torch.empty(max(nbytes, 1024), dtype=torch.uint8, device=x.device)
         probs = torch.empty(x.shape[0], dtype=torch.float32, device=x.device)
         N.check(N.lib().smz_dsn_forward(N.ptr(x), is_bf16, cu.ctypes.data_as(C.c_void_p), len(lengths), C.byref(st), 1,
                                         N.ptr(probs), N.ptr(ws), ws.numel(), N.current_stream()))

@@ -12,6 +12,7 @@ import torch
 
 from .. import _native as N
 from ..dense import gemm
+from ._packed import ShadowCache  # noqa: F401 (earlier import location)
 
 
 class LstmSeq(C.Structure):
@@ -32,25 +33,6 @@ class LstmDecode(C.Structure):
 def _off(t, elems):
     """device address of t.data_ptr() + elems elements (None stays None)."""
     return None if t is None else t.data_ptr() + elems * t.element_size()
-
-
-class ShadowCache:
-    """bf16 / transposed copies of parameters for the kernels.  ``fresh=True`` (training forwards) always rebuilds and
-    leaves the entry dirty: an optimizer step follows, and fused optimizers update parameters without bumping
-    ``Tensor._version``.  Inference calls reuse an entry until a version / storage changes or a training forward
-    happened in between."""
-
-    def __init__(self):
-        self._store = {}
-
-    def get(self, key, params, build, fresh=False):
-        tag = tuple((p.data_ptr(), p._version) for p in params)
-        ent = self._store.get(key)
-        if fresh or ent is None or ent[0] is None or ent[0] != tag:
-            with torch.no_grad():
-                ent = (None if fresh else tag, build())
-            self._store[key] = ent
-        return ent[1]
 
 
 def _sync_ws(device):
@@ -91,7 +73,7 @@ class _LstmLayerFn(torch.autograd.Function):
         cache, key, nd, H = meta
         dirs = [flat[4 * i: 4 * i + 4] for i in range(nd)]
         training = any(ctx.needs_input_grad)
-        sh = cache.get(key, flat, lambda: _LayerShadow(dirs), fresh=training)
+        sh = cache.get(flat, lambda: _LayerShadow(dirs), key=key, fresh=training)
         B, T, dev = x.shape[0], x.shape[1], x.device
         xb = _bf(x).reshape(B * T, -1)
         pre = gemm(xb, sh.w_ih, bias=sh.bias)                                     # [B*T, nd*4H]
@@ -206,7 +188,7 @@ class _DecodeFn(torch.autograd.Function):
         cache, key, T, H = meta
         p0, p1 = flat[:4], flat[4:]
         training = any(ctx.needs_input_grad)
-        sh = cache.get(key, flat, lambda: _DecodeShadow(p0, p1), fresh=training)
+        sh = cache.get(flat, lambda: _DecodeShadow(p0, p1), key=key, fresh=training)
         dev, B = h_init.device, h_init.shape[1]
         f32 = dict(dtype=torch.float32, device=dev)
         hi, ci = h_init.detach().float().contiguous(), c_init.detach().float().contiguous()

@@ -15,7 +15,8 @@ import torch.nn as nn
 
 from .. import _native as N
 from ..dense import linear
-from .lstm_stack import ShadowCache, lstm_decode, lstm_stack
+from ._packed import NativeModule
+from .lstm_stack import lstm_decode, lstm_stack
 
 
 class NoiseSource:
@@ -48,14 +49,13 @@ def _head1(x, lin):
     return (x * lin.weight.reshape(1, -1)).sum(-1, keepdim=True) + lin.bias
 
 
-class sLSTM(nn.Module):
+class sLSTM(NativeModule):
     def __init__(self, input_size=1024, hidden_size=1024, num_layers=2):
         """Selector LSTM"""
         super().__init__()
         self.lstm = nn.LSTM(input_size=input_size, hidden_size=hidden_size, num_layers=num_layers, bidirectional=True)
         self.out = nn.Linear(hidden_size * 2, 1)
         self.sig = nn.Sigmoid()
-        self._cache = ShadowCache()
 
     def forward(self, x):
         """x: (seq_len, batch_size, input_size) -> scores: (seq_len, batch_size, 1)"""
@@ -64,14 +64,13 @@ class sLSTM(nn.Module):
         return torch.sigmoid(_head1(y, self.out)).transpose(0, 1)
 
 
-class eLSTM(nn.Module):
+class eLSTM(NativeModule):
     def __init__(self, input_size=1024, hidden_size=2048, num_layers=2):
         """Encoder LSTM"""
         super().__init__()
         self.lstm = nn.LSTM(input_size=input_size, hidden_size=hidden_size, num_layers=num_layers, bidirectional=False)
         self.mu = nn.Linear(hidden_size, hidden_size)
         self.logvar = nn.Linear(hidden_size, hidden_size)
-        self._cache = ShadowCache()
 
     def forward(self, x):
         """x: (seq_len, batch_size, input_size) -> (h_mu, h_logvar), c_last: each (num_layers, batch_size, hidden_size)"""
@@ -84,13 +83,12 @@ class eLSTM(nn.Module):
         return (h_mu, h_logvar), c_last
 
 
-class dLSTM(nn.Module):
+class dLSTM(NativeModule):
     def __init__(self, input_size=1024, hidden_size=2048, num_layers=2):
         """Decoder LSTM"""
         super().__init__()
         self.lstm = nn.LSTM(input_size=hidden_size, hidden_size=hidden_size, num_layers=num_layers, bidirectional=False)
         self.recons = nn.Linear(hidden_size, input_size)
-        self._cache = ShadowCache()
 
     def forward_step(self, x_prev, h_prev, c_prev):
         """Decode one sequence step: x_prev (1, B, H), h_prev/c_prev (num_layers, B, H) -> x_next, (h_next, c_next)."""
@@ -150,13 +148,12 @@ class Summarizer(nn.Module):
         return x_hat, (h_mu, h_logvar), scores
 
 
-class cLSTM(nn.Module):
+class cLSTM(NativeModule):
     def __init__(self, input_size=1024, hidden_size=1024, num_layers=2):
         """Discriminator as a classifier LSTM"""
         super().__init__()
         self.lstm = nn.LSTM(input_size=input_size, hidden_size=hidden_size, num_layers=num_layers, bidirectional=False)
         self.out = nn.Sequential(nn.Linear(hidden_size, 1), nn.Sigmoid())
-        self._cache = ShadowCache()
 
     def forward(self, x):
         """x: (seq_len, B, input_size) -> probs (B, 1), h_last (B, hidden_size)"""

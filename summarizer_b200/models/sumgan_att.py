@@ -15,9 +15,9 @@ import torch
 import torch.nn as nn
 
 from .. import _native as N
+from ._packed import NativeModule, Workspace, packed_input, score_sequences, workspace_bytes
 from .sumgan import GAN, SumGANTrainer
 from .transformer import encoder_copies, encoder_params, f32, layer_table
-from .vasnet import _cu_seqlens, _Workspace
 
 
 class SelectorParams(C.Structure):
@@ -26,7 +26,7 @@ class SelectorParams(C.Structure):
                 ("eps", C.c_float), ("out_w", C.c_void_p), ("out_b", C.c_void_p)]
 
 
-class Transformer(nn.Module):
+class Transformer(NativeModule):
     """Selector: transformer encoder + Linear/Sigmoid per frame (sumgan_att.py:20-46)."""
 
     def __init__(self, input_size=1024, encoder_layers=4, attention_heads=8, epsilon=1e-5):
@@ -39,9 +39,7 @@ class Transformer(nn.Module):
         self.transformer_encoder = nn.TransformerEncoder(self.transformer_encoder_layer, num_layers=encoder_layers,
                                                          norm=self.layer_norm)
         self.out = nn.Sequential(nn.Linear(input_size, 1), nn.Sigmoid())
-        self._shadow = None
-        self._shadow_key = None
-        self._ws = _Workspace()
+        self._ws = Workspace()
 
     def native_covered(self):
         """True when the sm_100a kernels implement this configuration (1024-d input, 4 heads of width 256 or 8 of width
@@ -49,19 +47,14 @@ class Transformer(nn.Module):
         return self.input_size == 1024 and self.attention_heads in (4, 8) and len(self.transformer_encoder.layers) >= 1
 
     def _weights(self):
-        """bfloat16 copies of the encoder matrices and the parameter structs, cached as models/transformer.py
-        ``Transformer._weights`` caches them: until a parameter's storage or version changes, marked dirty by a
-        training-mode forward (the library's Adam updates parameters in place without bumping ``_version``) and by
-        ``Trainer._invalidate_shadows`` through ``_shadow_key``."""
+        """The parameter struct over the kernels' weight copies (cached in ``self._cache``)."""
         layers = list(self.transformer_encoder.layers)
         lin = self.out[0]
         ps = encoder_params(layers) + [self.layer_norm.weight, self.layer_norm.bias, lin.weight, lin.bias]
-        key = tuple((p.data_ptr(), p._version) for p in ps) + (float(self.layer_norm.eps),)
-        if self._shadow_key is None or key != self._shadow_key:
-            self._shadow = dict(layers=encoder_copies(layers), ln_g=f32(self.layer_norm.weight),
-                                ln_b=f32(self.layer_norm.bias), out_w=f32(lin.weight).reshape(-1), out_b=f32(lin.bias))
-            self._shadow_key = key
-        sh = self._shadow
+        sh = self._cache.get(ps, lambda: dict(layers=encoder_copies(layers), ln_g=f32(self.layer_norm.weight),
+                                              ln_b=f32(self.layer_norm.bias), out_w=f32(lin.weight).reshape(-1),
+                                              out_b=f32(lin.bias)),
+                             config=(float(self.layer_norm.eps),))
         arr = layer_table(sh["layers"])
         st = SelectorParams(C.addressof(arr), int(self.attention_heads), sh["ln_g"].data_ptr(), sh["ln_b"].data_ptr(),
                             float(self.layer_norm.eps), sh["out_w"].data_ptr(), sh["out_b"].data_ptr())
@@ -70,20 +63,12 @@ class Transformer(nn.Module):
     def score_packed(self, x, lengths):
         """Inference over a ragged batch: ``x`` packed [sum T, 1024] (float32 or bfloat16, device), ``lengths`` the
         per-video frame counts.  Returns float32 scores [sum T]; every video attends only to its own frames."""
-        N.require_device()
         if not self.native_covered():
             raise N.NativeError("score_packed: the sm_100a kernels cover 1024-d input with 4 or 8 attention heads only")
-        if x.dtype not in (torch.float32, torch.bfloat16):
-            x = x.float()
-        x = x.contiguous()
-        cu = _cu_seqlens(lengths)
-        assert x.shape == (int(cu[-1]), self.input_size)
+        x, cu, is_bf16 = packed_input(x, lengths, self.input_size)
         st, arr = self._weights()           # arr: the layer table st points at, alive for the call
         cu_p = cu.ctypes.data_as(C.c_void_p)
-        is_bf16 = int(x.dtype == torch.bfloat16)
-        nbytes = C.c_int64(0)
-        N.check(N.lib().smz_transformer_workspace_bytes(cu_p, len(lengths), is_bf16, C.byref(nbytes)))
-        ws = self._ws.get(nbytes.value, x.device)
+        ws = self._ws.get(workspace_bytes(N.lib().smz_transformer_workspace_bytes, cu_p, len(lengths), is_bf16), x.device)
         scores = torch.empty(x.shape[0], dtype=torch.float32, device=x.device)
         N.check(N.lib().smz_sumgan_att_selector_forward(N.ptr(x), is_bf16, cu_p, len(lengths), C.byref(st),
                                                         len(self.transformer_encoder.layers), N.ptr(scores), N.ptr(ws),
@@ -93,13 +78,10 @@ class Transformer(nn.Module):
     def forward(self, x):
         """x: (seq_len, batch_size, input_size) -> scores: (seq_len, batch_size, 1)"""
         if self.training:
-            self._shadow_key = None          # an optimizer step may follow: the weight copies must be rebuilt
+            self._cache.clear()              # an optimizer step may follow: the weight copies must be rebuilt
         builds_graph = torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in self.parameters()))
         if x.is_cuda and not self.training and not builds_graph and self.native_covered():
-            seq_len, batch_size, _ = x.shape
-            packed = x.permute(1, 0, 2).reshape(batch_size * seq_len, self.input_size)
-            s = self.score_packed(packed, [seq_len] * batch_size)
-            return s.view(batch_size, seq_len, 1).permute(1, 0, 2)
+            return score_sequences(self.score_packed, x)
         return self.out(self.transformer_encoder(x))
 
 
@@ -174,16 +156,9 @@ class SumGANAttTrainer(SumGANTrainer):
         self.log.debug("Discriminator params: {}".format(sum([_.numel() for _ in model.gan.parameters()])))
         return model
 
-    def _score_keys(self, keys):
-        """All test videos in ONE packed native call (ragged batch) instead of one forward per video."""
+    def _packed_scorer(self):
         sel = self.model.summarizer.selector
-        if not sel.native_covered() or not self.hps.use_cuda:
-            return super()._score_keys(keys)
-        feats = [self._video_tensors(k)[0][:, 0] for k in keys]
-        lengths = [f.shape[0] for f in feats]
-        with torch.no_grad():
-            packed = sel.score_packed(torch.cat(feats), lengths)
-        return list(torch.split(packed, lengths))
+        return sel if sel.native_covered() and self.hps.use_cuda else None
 
     # ---- losses (sumgan_att.py:171-193) ----------------------------------------------------------------------
     def loss_ae(self, x, x_hat):

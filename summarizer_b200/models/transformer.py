@@ -16,7 +16,7 @@ import torch.nn as nn
 
 from .. import _native as N
 from . import Trainer
-from .vasnet import _cu_seqlens, _Workspace
+from ._packed import NativeModule, Workspace, packed_input, score_sequences, workspace_bytes
 
 
 class TransformerLayerParams(C.Structure):
@@ -49,11 +49,10 @@ def b16(t):
 
 def encoder_copies(layers):
     """Per layer, the smz_transformer_layer tensors: bfloat16 copies of the matrices, float32 vectors."""
-    with torch.no_grad():
-        return [(b16(L.self_attn.in_proj_weight), f32(L.self_attn.in_proj_bias), b16(L.self_attn.out_proj.weight),
-                 f32(L.self_attn.out_proj.bias), b16(L.linear1.weight), f32(L.linear1.bias), b16(L.linear2.weight),
-                 f32(L.linear2.bias), f32(L.norm1.weight), f32(L.norm1.bias), f32(L.norm2.weight), f32(L.norm2.bias))
-                for L in layers]
+    return [(b16(L.self_attn.in_proj_weight), f32(L.self_attn.in_proj_bias), b16(L.self_attn.out_proj.weight),
+             f32(L.self_attn.out_proj.bias), b16(L.linear1.weight), f32(L.linear1.bias), b16(L.linear2.weight),
+             f32(L.linear2.bias), f32(L.norm1.weight), f32(L.norm1.bias), f32(L.norm2.weight), f32(L.norm2.bias))
+            for L in layers]
 
 
 def layer_table(copies):
@@ -73,7 +72,7 @@ def sincos_table(max_length, width):
     return table
 
 
-class Transformer(nn.Module):
+class Transformer(NativeModule):
     def __init__(self, input_size=1024, encoder_layers=6, attention_heads=8, more_residuals=False, max_length=None,
                  pos_embed="simple", epsilon=1e-5, weight_init=None):
         super().__init__()
@@ -108,9 +107,7 @@ class Transformer(nn.Module):
                 init(layer.linear2.weight)
             init(self.k1.weight)
             init(self.k2.weight)
-        self._shadow = None
-        self._shadow_key = None
-        self._ws = _Workspace()
+        self._ws = Workspace()
 
     def native_covered(self):
         """True when the sm_100a kernels implement this configuration (1024-d input, 8 heads of width 128, at least one
@@ -118,50 +115,39 @@ class Transformer(nn.Module):
         return self.input_size == 1024 and self.attention_heads == 8 and len(self.transformer_encoder.layers) >= 1
 
     def _weights(self):
-        """bfloat16 copies of the encoder / k1 matrices and the parameter structs, cached until a parameter's storage or
-        version changes (``load_state_dict``, ``.cuda()``).  A training-mode forward marks the cache dirty (the library's
-        Adam updates parameters in place without bumping ``_version``), and so does ``Trainer._invalidate_shadows``,
-        which reaches this module through ``_shadow_key``.  Only ``transformer_encoder.layers.*`` run: the top-level
-        ``transformer_encoder_layer`` is a template the encoder deep-copied and is never read."""
+        """The parameter structs over the kernels' weight copies (``_build_weights``, cached in ``self._cache``).  Only
+        ``transformer_encoder.layers.*`` run: the top-level ``transformer_encoder_layer`` is a template the encoder
+        deep-copied and is never read."""
         layers = list(self.transformer_encoder.layers)
         ps = encoder_params(layers)
         ps += [self.layer_norm.weight, self.layer_norm.bias, self.k1.weight, self.k1.bias, self.k2.weight, self.k2.bias]
-        key = tuple((p.data_ptr(), p._version) for p in ps) + (bool(self.more_residuals), float(self.epsilon))
-        if self._shadow_key is None or key != self._shadow_key:
-            per_layer = encoder_copies(layers)
-            with torch.no_grad():
-                ln_g, ln_b = f32(self.layer_norm.weight), f32(self.layer_norm.bias)
-                w2, b2 = f32(self.k2.weight).reshape(-1), f32(self.k2.bias)
-                head_gw = (ln_g * w2).contiguous()
-                head_c = torch.stack([head_gw.sum(), (ln_b * w2).sum() + b2[0]]).contiguous()
-                self._shadow = dict(layers=per_layer, ln_g=ln_g, ln_b=ln_b, k1_w=b16(self.k1.weight), k1_b=f32(self.k1.bias),
-                                    head_gw=head_gw, head_c=head_c)
-            self._shadow_key = key
-        sh = self._shadow
+        sh = self._cache.get(ps, lambda: self._build_weights(layers), config=(bool(self.more_residuals), float(self.epsilon)))
         arr = layer_table(sh["layers"])
         st = TransformerParams(C.addressof(arr), sh["ln_g"].data_ptr(), sh["ln_b"].data_ptr(), float(self.epsilon),
                                int(bool(self.more_residuals)), sh["k1_w"].data_ptr(), sh["k1_b"].data_ptr(),
                                sh["head_gw"].data_ptr(), sh["head_c"].data_ptr())
         return st, arr
 
+    def _build_weights(self, layers):
+        """bfloat16 copies of the encoder / k1 matrices, float32 vectors and the folded regressor head."""
+        per_layer = encoder_copies(layers)
+        ln_g, ln_b = f32(self.layer_norm.weight), f32(self.layer_norm.bias)
+        w2, b2 = f32(self.k2.weight).reshape(-1), f32(self.k2.bias)
+        head_gw = (ln_g * w2).contiguous()
+        head_c = torch.stack([head_gw.sum(), (ln_b * w2).sum() + b2[0]]).contiguous()
+        return dict(layers=per_layer, ln_g=ln_g, ln_b=ln_b, k1_w=b16(self.k1.weight), k1_b=f32(self.k1.bias),
+                    head_gw=head_gw, head_c=head_c)
+
     def score_packed(self, x, lengths):
         """Inference over a ragged batch: ``x`` packed [sum T, 1024] (float32 or bfloat16, device, positional embeddings
         already added), ``lengths`` the per-video frame counts.  Returns float32 scores [sum T]; every video attends
         only to its own frames."""
-        N.require_device()
         if not self.native_covered():
             raise N.NativeError("score_packed: the sm_100a kernels cover 1024-d input with 8 attention heads only")
-        if x.dtype not in (torch.float32, torch.bfloat16):
-            x = x.float()
-        x = x.contiguous()
-        cu = _cu_seqlens(lengths)
-        assert x.shape == (int(cu[-1]), self.input_size)
+        x, cu, is_bf16 = packed_input(x, lengths, self.input_size)
         st, arr = self._weights()           # arr: the layer table st points at, alive for the call
         cu_p = cu.ctypes.data_as(C.c_void_p)
-        is_bf16 = int(x.dtype == torch.bfloat16)
-        nbytes = C.c_int64(0)
-        N.check(N.lib().smz_transformer_workspace_bytes(cu_p, len(lengths), is_bf16, C.byref(nbytes)))
-        ws = self._ws.get(nbytes.value, x.device)
+        ws = self._ws.get(workspace_bytes(N.lib().smz_transformer_workspace_bytes, cu_p, len(lengths), is_bf16), x.device)
         scores = torch.empty(x.shape[0], dtype=torch.float32, device=x.device)
         N.check(N.lib().smz_transformer_forward(N.ptr(x), is_bf16, cu_p, len(lengths), C.byref(st),
                                                 len(self.transformer_encoder.layers), N.ptr(scores), N.ptr(ws), ws.numel(),
@@ -172,7 +158,7 @@ class Transformer(nn.Module):
         """x: (seq_len, batch_size, input_size) -> y: (seq_len, batch_size, 1)"""
         seq_len, batch_size, _ = x.shape
         if self.training:
-            self._shadow_key = None          # an optimizer step may follow: the weight copies must be rebuilt
+            self._cache.clear()              # an optimizer step may follow: the weight copies must be rebuilt
         if self.max_length is not None:
             assert self.max_length >= seq_len, "input sequence has higher length than max_length"
             if self.pos_embed_type == "simple":
@@ -182,9 +168,7 @@ class Transformer(nn.Module):
             x += pe.unsqueeze(1)                              # in place on the caller's tensor, as upstream (:84,:86)
         builds_graph = torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in self.parameters()))
         if x.is_cuda and not self.training and not builds_graph and self.native_covered():
-            packed = x.permute(1, 0, 2).reshape(batch_size * seq_len, self.input_size)
-            s = self.score_packed(packed, [seq_len] * batch_size)
-            return s.view(batch_size, seq_len, 1).permute(1, 0, 2)
+            return score_sequences(self.score_packed, x)
         encoder_out = self.transformer_encoder(x)
         if self.more_residuals:
             encoder_out = encoder_out + x
@@ -201,16 +185,9 @@ class TransformerTrainer(Trainer):
                            pos_embed=ep.get("pos_embed", "simple"), epsilon=float(ep.get("epsilon", 1e-5)),
                            weight_init=ep.get("weight_init", None))
 
-    def _score_keys(self, keys):
-        """All test videos in ONE packed native call (ragged batch) instead of one forward per video."""
+    def _packed_scorer(self):
         m = self.model
-        if getattr(m, "max_length", None) is not None or not m.native_covered() or not self.hps.use_cuda:
-            return super()._score_keys(keys)
-        feats = [self._video_tensors(k)[0][:, 0] for k in keys]
-        lengths = [f.shape[0] for f in feats]
-        with torch.no_grad():
-            packed = m.score_packed(torch.cat(feats), lengths)
-        return list(torch.split(packed, lengths))
+        return m if m.max_length is None and m.native_covered() and self.hps.use_cuda else None
 
     def train(self, fold):
         return self._train_supervised(fold)

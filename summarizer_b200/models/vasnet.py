@@ -8,6 +8,7 @@ files load unchanged (``layer_norm.{weight,bias}``, ``{K,Q,V,attention_head_proj
 tensor cores are derived on the fly and never saved.  There is no CPU / eager fallback.
 """
 import ctypes as C
+import functools
 import math
 
 import numpy as np
@@ -16,6 +17,8 @@ import torch.nn as nn
 import torch.nn.init as init
 
 from .. import _native as N
+from ._packed import NativeModule, Workspace, cu_seqlens, packed_input, score_sequences, workspace_bytes
+from ._packed import Workspace as _Workspace, cu_seqlens as _cu_seqlens  # noqa: F401 (earlier import location)
 
 
 class VasnetParams(C.Structure):
@@ -32,25 +35,7 @@ SPLIT = 4      # SMZ_VASNET_SPLIT: OR into `training` of smz_vasnet_workspace_by
 LO_KEYS = ("wqk_lo", "wv_lo", "wo_lo", "w1_lo")
 
 
-def _cu_seqlens(lengths):
-    cu = np.zeros(len(lengths) + 1, dtype=np.int32)
-    np.cumsum(np.asarray(lengths, dtype=np.int64), out=cu[1:])
-    return cu
-
-
-class _Workspace:
-    """Grow-only device work buffer, one per (device, purpose)."""
-
-    def __init__(self):
-        self.buf = None
-
-    def get(self, nbytes, device):
-        if self.buf is None or self.buf.numel() < nbytes or self.buf.device != device:
-            self.buf = torch.empty(max(int(nbytes), 1024), dtype=torch.uint8, device=device)
-        return self.buf
-
-
-class VASNet(nn.Module):
+class VASNet(NativeModule):
     def __init__(self, input_size=1024, max_length=None, pos_embed="simple", ignore_self=False,
                  attention_aperture=None, scale=None, epsilon=1e-6, weight_init="xavier", precision="bf16"):
         """Reference constructor (vasnet.py:18-21) + ``precision``: "bf16" (default: bf16 / float16 tensor-core operands,
@@ -106,89 +91,87 @@ class VASNet(nn.Module):
         init.constant_(self.k1.bias, 0.1)
         init.constant_(self.k2.bias, 0.1)
 
-        self._shadow = None
-        self._shadow_key = None
         self._status = None
-        self._ws = _Workspace()
+        self._ws = Workspace()
 
     # ---------------------------------------------------------------------------------------------
     def _weights(self, inference=True, fast=True):
-        """bfloat16 shadow copies + the parameter struct.  A training forward (``inference=False``) ALWAYS rebuilds
-        them and leaves the cache marked dirty: an optimizer step follows, and fused optimizers update the parameters
-        without bumping ``Tensor._version``, so a version key cannot be trusted across a step.  Inference calls reuse
-        the copies until a parameter's version / storage changes (``load_state_dict``, ``.cuda()``) or a training
-        forward happened in between.  The folded head constants are only derived for inference (the training path
-        keeps the separate head kernel)."""
+        """The kernels' weight copies (``_build_weights``, cached in ``self._cache``; a training forward,
+        ``inference=False``, rebuilds them) and the parameter struct over them.  The fast inference path's fields are set
+        when ``fast`` and its weights allow it."""
         ps = (self.Q.weight, self.K.weight, self.V.weight, self.attention_head_projection.weight,
               self.k1.weight, self.k1.bias, self.k2.weight, self.k2.bias, self.layer_norm.weight,
               self.layer_norm.bias)
-        key = tuple((p.data_ptr(), p._version) for p in ps) + (self.precision,)
-        if self.precision == "fp32":
-            fast = False                     # the folded 16-bit fast path is the bf16 mode's
-        if not inference or self._shadow_key is None or key != self._shadow_key:
-            with torch.no_grad():
-                big = (self.Q.weight, self.K.weight, self.V.weight, self.attention_head_projection.weight, self.k1.weight)
-                lo = None
-                if self.precision == "fp32":
-                    # float32-accurate mode: hi + lo bf16 planes of the five matrices in one launch
-                    src_t = [t.detach().float().contiguous() for t in big]
-                    flat = torch.empty(2, 5 * 1024 * 1024, dtype=torch.bfloat16, device=big[0].device)
-                    src = (C.c_void_p * 5)(*(t.data_ptr() for t in src_t))
-                    dst = (C.c_void_p * 5)(*(flat[0].data_ptr() + 2 * 1024 * 1024 * i for i in range(5)))
-                    dlo = (C.c_void_p * 5)(*(flat[1].data_ptr() + 2 * 1024 * 1024 * i for i in range(5)))
-                    cnt = (C.c_int64 * 5)(*([1024 * 1024] * 5))
-                    N.check(N.lib().smz_split_bf16_multi(src, dst, dlo, cnt, 5, N.current_stream()))
-                    w, wl = flat[0].view(5 * 1024, 1024), flat[1].view(5 * 1024, 1024)
-                    wqk, wv, wo, w1 = w[:2048], w[2048:3072], w[3072:4096], w[4096:]
-                    lo = dict(wqk_lo=wl[:2048], wv_lo=wl[2048:3072], wo_lo=wl[3072:4096], w1_lo=wl[4096:])
-                elif all(t.is_cuda and t.dtype == torch.float32 and t.is_contiguous() for t in big):
-                    # one launch: [Q;K] | V | O | k1 -> one bf16 buffer (no fp32 concatenation, no cast kernel per tensor)
-                    flat = torch.empty(5 * 1024 * 1024, dtype=torch.bfloat16, device=big[0].device)
-                    src = (C.c_void_p * 5)(*(t.data_ptr() for t in big))
-                    dst = (C.c_void_p * 5)(*(flat.data_ptr() + 2 * 1024 * 1024 * i for i in range(5)))
-                    cnt = (C.c_int64 * 5)(*([1024 * 1024] * 5))
-                    N.check(N.lib().smz_cvt_bf16_multi(src, dst, cnt, 5, N.current_stream()))
-                    w = flat.view(5 * 1024, 1024)
-                    wqk, wv, wo, w1 = w[:2048], w[2048:3072], w[3072:4096], w[4096:]
-                else:
-                    wqk = torch.cat([self.Q.weight, self.K.weight], 0).to(torch.bfloat16).contiguous()
-                    wv, wo, w1 = (t.to(torch.bfloat16).contiguous() for t in big[2:])
-                sh = dict(
-                    wqk=wqk, wv=wv, wo=wo, w1=w1,
-                    b1=self.k1.bias.float().contiguous(), w2=self.k2.weight.float().reshape(-1).contiguous(),
-                    b2=self.k2.bias.float().contiguous(), ln_g=self.layer_norm.weight.float().contiguous(),
-                    ln_b=self.layer_norm.bias.float().contiguous())
-                if lo is not None:
-                    sh.update(lo)
-            self._shadow, self._shadow_key = sh, (key if inference else None)
-        sh = self._shadow
-        if inference and "head_gw" not in sh:
-            with torch.no_grad():   # regressor head folded into the k1 epilogue: z = rstd * (sum h*gw - mean * c0) + c1
-                sh["head_gw"] = (sh["ln_g"] * sh["w2"]).contiguous()
-                sh["head_c"] = torch.stack([sh["head_gw"].sum(), (sh["ln_b"] * sh["w2"]).sum() + sh["b2"][0]]).contiguous()
-                # first LayerNorm folded into k1: W1.LN(y) + b1 = rstd * (W1g.y - mean * rowsum(W1g)) + (W1.ln_b + b1)
-                w1 = self.k1.weight.float()
-                sh["w1g"] = (w1 * sh["ln_g"][None, :]).to(torch.float16).contiguous()       # float16: y is handed over as float16
-                sh["ln_c"] = sh["w1g"].float().sum(1).contiguous()
-                sh["b1f"] = (w1 @ sh["ln_b"] + sh["b1"]).contiguous()
-                # folded projections of the fast path (products in float32): rows 0..1023 = Wo Wv, 1024..2047 = Wk^T Wq.
-                # The fast path is only offered when 16-bit floats hold them well (no overflow, the largest entries far
-                # above the float16 subnormal range)
-                wq, wk, wv, wo = (t.detach().float() for t in (self.Q.weight, self.K.weight, self.V.weight,
-                                                               self.attention_head_projection.weight))
-                gv = torch.cat([wo @ wv, wk.t() @ wq], 0)
-                amax = torch.stack([gv[:1024].abs().max(), gv[1024:].abs().max(), (w1 * sh["ln_g"][None, :]).abs().max()])
-                sh["fast_ok"] = bool((torch.isfinite(amax) & (amax < 6e4) & (amax > 1e-3)).all().item())
-                sh["wgv"] = gv.to(torch.bfloat16).contiguous()
-                sh["wgv16"] = gv.to(torch.float16).contiguous()
+        sh = self._cache.get(ps, lambda: self._build_weights(inference), config=(self.precision,), fresh=not inference)
+        # the folded 16-bit fast path is the bf16 mode's
+        fast = inference and fast and self.precision != "fp32" and sh["fast_ok"]
         st = VasnetParams(*(sh[k].data_ptr() for k in ("wqk", "wv", "wo", "w1", "b1", "w2", "b2", "ln_g", "ln_b")),
                           float(self.scale), float(self.epsilon),
                           -1 if self.aperture is None else int(self.aperture), int(bool(self.ignore_self)),
                           *((sh[k].data_ptr() if inference else None) for k in ("head_gw", "head_c", "w1g", "ln_c", "b1f")),
-                          *((sh[k].data_ptr() if (inference and fast and sh["fast_ok"]) else None) for k in ("wgv", "wgv16")),
-                          self._status_word(sh["ln_g"].device).data_ptr() if (inference and fast and sh["fast_ok"]) else None,
+                          *((sh[k].data_ptr() if fast else None) for k in ("wgv", "wgv16")),
+                          self._status_word(sh["ln_g"].device).data_ptr() if fast else None,
                           *((sh[k].data_ptr() if k in sh else None) for k in LO_KEYS))
         return sh, st
+
+    def _build_weights(self, inference):
+        """bfloat16 copies of the matrices (plus their lo planes in the float32-accurate mode) and float32 vectors.  The
+        folded head constants and the fast path's folded projections are only derived for inference (the training path
+        keeps the separate head kernel)."""
+        big = (self.Q.weight, self.K.weight, self.V.weight, self.attention_head_projection.weight, self.k1.weight)
+        lo = None
+        if self.precision == "fp32":
+            # float32-accurate mode: hi + lo bf16 planes of the five matrices in one launch
+            src_t = [t.detach().float().contiguous() for t in big]
+            flat = torch.empty(2, 5 * 1024 * 1024, dtype=torch.bfloat16, device=big[0].device)
+            src = (C.c_void_p * 5)(*(t.data_ptr() for t in src_t))
+            dst = (C.c_void_p * 5)(*(flat[0].data_ptr() + 2 * 1024 * 1024 * i for i in range(5)))
+            dlo = (C.c_void_p * 5)(*(flat[1].data_ptr() + 2 * 1024 * 1024 * i for i in range(5)))
+            cnt = (C.c_int64 * 5)(*([1024 * 1024] * 5))
+            N.check(N.lib().smz_split_bf16_multi(src, dst, dlo, cnt, 5, N.current_stream()))
+            w, wl = flat[0].view(5 * 1024, 1024), flat[1].view(5 * 1024, 1024)
+            wqk, wv, wo, w1 = w[:2048], w[2048:3072], w[3072:4096], w[4096:]
+            lo = dict(wqk_lo=wl[:2048], wv_lo=wl[2048:3072], wo_lo=wl[3072:4096], w1_lo=wl[4096:])
+        elif all(t.is_cuda and t.dtype == torch.float32 and t.is_contiguous() for t in big):
+            # one launch: [Q;K] | V | O | k1 -> one bf16 buffer (no fp32 concatenation, no cast kernel per tensor)
+            flat = torch.empty(5 * 1024 * 1024, dtype=torch.bfloat16, device=big[0].device)
+            src = (C.c_void_p * 5)(*(t.data_ptr() for t in big))
+            dst = (C.c_void_p * 5)(*(flat.data_ptr() + 2 * 1024 * 1024 * i for i in range(5)))
+            cnt = (C.c_int64 * 5)(*([1024 * 1024] * 5))
+            N.check(N.lib().smz_cvt_bf16_multi(src, dst, cnt, 5, N.current_stream()))
+            w = flat.view(5 * 1024, 1024)
+            wqk, wv, wo, w1 = w[:2048], w[2048:3072], w[3072:4096], w[4096:]
+        else:
+            wqk = torch.cat([self.Q.weight, self.K.weight], 0).to(torch.bfloat16).contiguous()
+            wv, wo, w1 = (t.to(torch.bfloat16).contiguous() for t in big[2:])
+        sh = dict(
+            wqk=wqk, wv=wv, wo=wo, w1=w1,
+            b1=self.k1.bias.float().contiguous(), w2=self.k2.weight.float().reshape(-1).contiguous(),
+            b2=self.k2.bias.float().contiguous(), ln_g=self.layer_norm.weight.float().contiguous(),
+            ln_b=self.layer_norm.bias.float().contiguous())
+        if lo is not None:
+            sh.update(lo)
+        if not inference:
+            return sh
+        # regressor head folded into the k1 epilogue: z = rstd * (sum h*gw - mean * c0) + c1
+        sh["head_gw"] = (sh["ln_g"] * sh["w2"]).contiguous()
+        sh["head_c"] = torch.stack([sh["head_gw"].sum(), (sh["ln_b"] * sh["w2"]).sum() + sh["b2"][0]]).contiguous()
+        # first LayerNorm folded into k1: W1.LN(y) + b1 = rstd * (W1g.y - mean * rowsum(W1g)) + (W1.ln_b + b1)
+        w1 = self.k1.weight.float()
+        sh["w1g"] = (w1 * sh["ln_g"][None, :]).to(torch.float16).contiguous()       # float16: y is handed over as float16
+        sh["ln_c"] = sh["w1g"].float().sum(1).contiguous()
+        sh["b1f"] = (w1 @ sh["ln_b"] + sh["b1"]).contiguous()
+        # folded projections of the fast path (products in float32): rows 0..1023 = Wo Wv, 1024..2047 = Wk^T Wq.
+        # The fast path is only offered when 16-bit floats hold them well (no overflow, the largest entries far
+        # above the float16 subnormal range)
+        wq, wk, wv, wo = (t.detach().float() for t in (self.Q.weight, self.K.weight, self.V.weight,
+                                                       self.attention_head_projection.weight))
+        gv = torch.cat([wo @ wv, wk.t() @ wq], 0)
+        amax = torch.stack([gv[:1024].abs().max(), gv[1024:].abs().max(), (w1 * sh["ln_g"][None, :]).abs().max()])
+        sh["fast_ok"] = bool((torch.isfinite(amax) & (amax < 6e4) & (amax > 1e-3)).all().item())
+        sh["wgv"] = gv.to(torch.bfloat16).contiguous()
+        sh["wgv16"] = gv.to(torch.float16).contiguous()
+        return sh
 
     def _status_word(self, device):
         """Device word the fast inference path ORs SMZ_VASNET_STATUS_* into (include/summarizer_b200.h)."""
@@ -215,20 +198,12 @@ class VASNet(nn.Module):
         kernels check on the fly; ``check=True`` reads the status word after the call (one synchronisation, as the
         reference's own ``.cpu()`` per video) and repeats the call on the exact path if a range was left.
         ``check=False`` leaves that to a later ``check_status()``; ``exact=True`` takes the exact path directly."""
-        N.require_device()
-        if x.dtype not in (torch.float32, torch.bfloat16):
-            x = x.float()
-        x = x.contiguous()
-        cu = _cu_seqlens(lengths)
-        assert x.shape == (int(cu[-1]), self.input_size)
+        x, cu, is_bf16 = packed_input(x, lengths, self.input_size)
         if self.precision == "fp32":
             return self._score_packed_split(x, lengths)
         _, st = self._weights(fast=not exact)
-        nbytes = C.c_int64(0)
         cu_p = cu.ctypes.data_as(C.c_void_p)
-        is_bf16 = int(x.dtype == torch.bfloat16)
-        N.check(N.lib().smz_vasnet_workspace_bytes(cu_p, len(lengths), 0, is_bf16, C.byref(nbytes)))
-        ws = self._ws.get(nbytes.value, x.device)
+        ws = self._ws.get(workspace_bytes(N.lib().smz_vasnet_workspace_bytes, cu_p, len(lengths), 0, is_bf16), x.device)
         scores = torch.empty(x.shape[0], dtype=torch.float32, device=x.device)
         N.check(N.lib().smz_vasnet_forward(N.ptr(x), is_bf16, cu_p, len(lengths), C.byref(st), 0, None, None, None,
                                            N.ptr(scores), N.ptr(ws), ws.numel(), N.current_stream()))
@@ -247,11 +222,8 @@ class VASNet(nn.Module):
             v1, rows = v0, 0
             while v1 < len(lengths) and (v1 == v0 or rows + lengths[v1] <= max_rows):
                 rows += int(lengths[v1]); v1 += 1
-            cu = _cu_seqlens(lengths[v0:v1])
-            cu_p = cu.ctypes.data_as(C.c_void_p)
-            nbytes = C.c_int64(0)
-            N.check(N.lib().smz_vasnet_workspace_bytes(cu_p, v1 - v0, 1 | SPLIT, is_bf16, C.byref(nbytes)))
-            ws = self._ws.get(nbytes.value, x.device)
+            cu_p = cu_seqlens(lengths[v0:v1]).ctypes.data_as(C.c_void_p)
+            ws = self._ws.get(workspace_bytes(N.lib().smz_vasnet_workspace_bytes, cu_p, v1 - v0, 1 | SPLIT, is_bf16), x.device)
             N.check(N.lib().smz_vasnet_forward(N.ptr(x[row0:row0 + rows]), is_bf16, cu_p, v1 - v0, C.byref(st), 1, None, None,
                                                None, N.ptr(scores[row0:row0 + rows]), N.ptr(ws), ws.numel(), N.current_stream()))
             v0, row0 = v1, row0 + rows
@@ -276,13 +248,10 @@ class VASNet(nn.Module):
                 xb += self.pos_embed(pos)
             else:
                 xb += self.pos_embed[:seq_len, :].repeat(1, batch_size).view(batch_size, seq_len, input_size).to(x.device)
-        packed = x.permute(1, 0, 2).reshape(batch_size * seq_len, input_size)
         if torch.is_grad_enabled() and (self.training or any(p.requires_grad for p in self.parameters())):
             from .vasnet_autograd import vasnet_apply
-            s = vasnet_apply(self, packed, [seq_len] * batch_size)
-        else:
-            s = self.score_packed(packed, [seq_len] * batch_size)
-        return s.view(batch_size, seq_len, 1).permute(1, 0, 2)
+            return score_sequences(functools.partial(vasnet_apply, self), x)
+        return score_sequences(self.score_packed, x)
 
 
 from . import Trainer  # noqa: E402
@@ -309,15 +278,8 @@ class VASNetTrainer(Trainer):
             model.cuda()
         return model
 
-    def _score_keys(self, keys):
-        """All test videos in ONE packed forward call (ragged batch) instead of one launch chain per video."""
-        if getattr(self.model, "max_length", None) is not None:
-            return super()._score_keys(keys)
-        feats = [self._video_tensors(k)[0][:, 0] for k in keys]
-        lengths = [f.shape[0] for f in feats]
-        with torch.no_grad():
-            packed = self.model.score_packed(torch.cat(feats), lengths)
-        return list(torch.split(packed, lengths))
+    def _packed_scorer(self):
+        return self.model if self.model.max_length is None else None
 
     def train(self, fold):
         return self._train_supervised(fold)

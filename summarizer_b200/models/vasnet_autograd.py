@@ -10,7 +10,8 @@ import ctypes as C
 import torch
 
 from .. import _native as N
-from .vasnet import LO_KEYS, SPLIT, VasnetParams, _cu_seqlens
+from ._packed import packed_input, workspace_bytes
+from .vasnet import LO_KEYS, SPLIT, VasnetParams
 
 
 class VasnetGrads(C.Structure):
@@ -45,18 +46,12 @@ def draw_keep_masks(lengths, device, generator=None):
 class _VasnetFunction(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, module, lengths, masks, wq, wk, wv, wo, w1, b1, w2, b2, ln_g, ln_b):
-        N.require_device()
-        x = x.contiguous()
-        if x.dtype not in (torch.float32, torch.bfloat16):
-            x = x.float()
-        cu = _cu_seqlens(lengths)
+        x, cu, is_bf16 = packed_input(x, lengths, 1024)
         cu_p = cu.ctypes.data_as(C.c_void_p)
-        is_bf16 = int(x.dtype == torch.bfloat16)
         sh, st = module._weights(inference=False)
-        nbytes = C.c_int64(0)
         split = SPLIT if module.precision == "fp32" else 0            # room for the activations' lo planes
-        N.check(N.lib().smz_vasnet_workspace_bytes(cu_p, len(lengths), 1 | split, is_bf16, C.byref(nbytes)))
-        ws = torch.empty(max(nbytes.value, 1024), dtype=torch.uint8, device=x.device)   # lives until backward
+        nbytes = workspace_bytes(N.lib().smz_vasnet_workspace_bytes, cu_p, len(lengths), 1 | split, is_bf16)
+        ws = torch.empty(max(nbytes, 1024), dtype=torch.uint8, device=x.device)   # lives until backward
         scores = torch.empty(x.shape[0], dtype=torch.float32, device=x.device)
         m_att, m_y, m_h = masks if masks is not None else (None, None, None)
         N.check(N.lib().smz_vasnet_forward(N.ptr(x), is_bf16, cu_p, len(lengths), C.byref(st), 1, N.ptr(m_att), N.ptr(m_y),
